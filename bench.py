@@ -18,6 +18,10 @@ resident ray batches.  Prints ONE JSON line.
   --optimizer      adds the fused Adam / AdamW update (SURVEY.md 8f next-2) to the step of both arms
   --regularisers   adds the interlevel + distortion losses (SURVEY.md 8f next-1) to the step of both arms
   --no-graph       launch the step eagerly (what a plain training loop does)
+  --dump-outputs DIR   after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32): the
+                   path's outputs and, for training configs, the loss and every gradient (the updated parameters with
+                   --optimizer).  Arrays beyond the 64 MB budget are replaced by a fixed, seeded sample of their
+                   elements; the inputs are seeded, so two builds can be compared output for output.
 
 `roofline` = the kernel with the largest share of the step (`rooflines` has every major kernel): algorithmic bytes or
 FLOPs per launch (DESIGN.md section 4) / CUDA-event duration, against MEASURED_PEAKS.json; `traffic` = DRAM bytes per
@@ -43,6 +47,7 @@ import torch  # noqa: E402
 METRIC = "train_step_rays_per_sec"
 UNIT = "rays/s"
 N_BATCHES = 4
+DUMP_BYTES = 60_000_000  # --dump-outputs budget: 64 MB with room for the .npy headers
 
 
 def load_peaks():
@@ -191,7 +196,7 @@ def run_reference(args, rank):
 
     w = WORKLOADS[args.config]
     sample = min(4096, w.rays)
-    steps, warmup = max(1, min(args.steps, 10)), max(1, min(args.warmup, 3))
+    steps, warmup = args.steps, args.warmup
     value, ms, cores, kind, cpu = cpu_reference_run(w, sample, steps, warmup, regularisers=args.regularisers,
                                                     optimizer=args.optimizer)
     what = ("the reference's own modules (oracle/_ref, unmodified) on its fp32 torch path" if kind == "reference"
@@ -306,6 +311,34 @@ def parity_at_config(model, w, rays_cpu, n_check: int = 4096):
     return report
 
 
+def step_outputs(out):
+    """The arrays of one forward's output dict, detached (holding them must not keep the autograd graph alive)."""
+    arrays = {k: v.detach() for k, v in out.items() if torch.is_tensor(v)}
+    arrays.update({f"weights_{i}": t.detach() for i, t in enumerate(out.get("weights_list", []))})
+    return arrays
+
+
+def dump_outputs(directory, arrays, seed: int = 0):
+    """Write {name: tensor} as directory/<name>.npy in float32, DUMP_BYTES in all.  The budget is shared smallest array
+    first; an array that gets k < numel elements is written as a seeded stratified sample of its flattened elements: one
+    element from each of k equal strides, in index order, so the same arguments always select the same elements."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    budget = DUMP_BYTES // 4
+    names = sorted(arrays, key=lambda k: arrays[k].numel())
+    for i, name in enumerate(names):
+        t = arrays[name].detach().float()
+        keep = min(t.numel(), budget // (len(names) - i))
+        budget -= keep
+        if keep < t.numel():
+            edges = torch.arange(keep + 1, dtype=torch.int64) * t.numel() // keep
+            u = torch.rand(keep, generator=torch.Generator().manual_seed(seed), dtype=torch.float64)
+            idx = edges[:-1] + (u * (edges[1:] - edges[:-1])).long()
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------------
 def run_b200(args, rank, world, local_rank):
     import torch.distributed as dist
@@ -373,6 +406,7 @@ def run_b200(args, rank, world, local_rank):
 
     def step():
         """One step on the rays in `cur`; leaves the step's scalar result in result['loss'] (device)."""
+        kept = result["outs"] = [] if args.dump_outputs else None  # the step's outputs, for --dump-outputs
         if not w.train:
             chunk = w.chunk or n
             acc = None
@@ -381,6 +415,8 @@ def run_b200(args, rank, world, local_rank):
                     out = model(bundle(cur, lo, min(lo + chunk, n)))
                     s = out["depth"].sum()
                     acc = s if acc is None else acc + s
+                    if kept is not None:
+                        kept.append(step_outputs(out))
             result["loss"] = acc
             return
         if opts is None:
@@ -396,6 +432,8 @@ def run_b200(args, rank, world, local_rank):
         else:
             arena.all_reduce()
         result["loss"] = loss.detach()
+        if kept is not None:
+            kept.append(step_outputs(out))
 
     def load_resident(i):
         cur_flat.copy_(resident_flat[i % n_batches], non_blocking=True)
@@ -488,6 +526,17 @@ def run_b200(args, rank, world, local_rank):
         run_step()
     torch.cuda.synchronize()
     ms_e2e = timed(load_host, args.steps, True)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the step receives from the last timed one (inference: every chunk's outputs, in ray order)
+        outs = result["outs"]
+        arrays = {k: torch.cat([o[k] for o in outs]) for k in outs[0]}
+        if w.train:
+            arrays["loss"] = result["loss"]
+            for name, p in used:
+                t = p if args.optimizer else p.grad
+                if t is not None:
+                    arrays[("param." if args.optimizer else "grad.") + name] = t
+        dump_outputs(args.dump_outputs, arrays)
 
     # ---- per-kernel durations from CUDA events on the launching stream (separate eager pass: the events add launch gaps)
     # (the two backward branches are serialised for this pass: overlapped kernels would time each other's contention)
@@ -643,7 +692,13 @@ def main():
                     help="add the fused Adam / AdamW update (SURVEY.md 8f next-2) to the step of both arms")
     ap.add_argument("--regularisers", action="store_true",
                     help="add the interlevel + distortion losses (SURVEY.md 8f next-1) to the step of both arms")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (and gradients or updated parameters) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of this repo's CUDA path (--impl b200)")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,6 +1,7 @@
 """Generate golden vectors by EXECUTING the reference's own fp32 torch path (container only).
 
-Usage:  python tests/golden/make_golden.py      (needs the read-only checkout at /root/reference)
+Usage:  python tests/golden/make_golden.py      (needs the reference modules: oracle/_ref or $NEURADAR_REFERENCE)
+        python tests/golden/make_golden.py --lidar-close-only   (runs without them, see gen_lidar_close)
 
 Writes tests/golden/*.npz.  The vectors pin `oracle/neuradar_oracle.py` (tests/test_oracle_golden.py)
 and are compared with the CUDA path on the GPU box, where the reference itself does not exist.
@@ -16,36 +17,37 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 import _ref_shim  # noqa: E402
 
-_ref_shim.install()
-
-from nerfstudio.cameras.rays import Frustums, RayBundle, RaySamples  # noqa: E402
-from nerfstudio.field_components.encodings import HashEncoding, SHEncoding  # noqa: E402
-from nerfstudio.field_components.field_heads import FieldHeadNames  # noqa: E402
-from nerfstudio.field_components.mlp import MLP  # noqa: E402
-from nerfstudio.field_components.neurad_encoding import (  # noqa: E402
-    ActorSettings,
-    NeuRADHashEncodingConfig,
-    StaticSettings,
-)
-from nerfstudio.fields.neurad_field import (  # noqa: E402
-    NeuRADField,
-    NeuRADFieldConfig,
-    NeuRADProposalField,
-    NeuRADProposalFieldConfig,
-)
-from nerfstudio.model_components.dynamic_actors import DynamicActors, DynamicActorsConfig  # noqa: E402
-from nerfstudio.model_components.ray_samplers import (  # noqa: E402
-    PDFSampler,
-    PowerSampler,
-    ProposalNetworkSampler,
-    UniformSampler,
-)
-from nerfstudio.model_components.renderers import (  # noqa: E402
-    AccumulationRenderer,
-    DepthRenderer,
-    FeatureRenderer,
-)
-from nerfstudio.utils.math import components_from_spherical_harmonics  # noqa: E402
+HAVE_REFERENCE = _ref_shim.available()
+if HAVE_REFERENCE:  # every generator except gen_lidar_close needs the reference
+    _ref_shim.install()
+    from nerfstudio.cameras.rays import Frustums, RayBundle, RaySamples  # noqa: E402
+    from nerfstudio.field_components.encodings import HashEncoding, SHEncoding  # noqa: E402
+    from nerfstudio.field_components.field_heads import FieldHeadNames  # noqa: E402
+    from nerfstudio.field_components.mlp import MLP  # noqa: E402
+    from nerfstudio.field_components.neurad_encoding import (  # noqa: E402
+        ActorSettings,
+        NeuRADHashEncodingConfig,
+        StaticSettings,
+    )
+    from nerfstudio.fields.neurad_field import (  # noqa: E402
+        NeuRADField,
+        NeuRADFieldConfig,
+        NeuRADProposalField,
+        NeuRADProposalFieldConfig,
+    )
+    from nerfstudio.model_components.dynamic_actors import DynamicActors, DynamicActorsConfig  # noqa: E402
+    from nerfstudio.model_components.ray_samplers import (  # noqa: E402
+        PDFSampler,
+        PowerSampler,
+        ProposalNetworkSampler,
+        UniformSampler,
+    )
+    from nerfstudio.model_components.renderers import (  # noqa: E402
+        AccumulationRenderer,
+        DepthRenderer,
+        FeatureRenderer,
+    )
+    from nerfstudio.utils.math import components_from_spherical_harmonics  # noqa: E402
 
 torch.set_grad_enabled(True)
 
@@ -503,7 +505,65 @@ def gen_radar_rays():
     save("radar_rays", **out)
 
 
+def _close_inputs(n, S, seed, scale):
+    """Sorted sample bins, lidar flags, hit distances (a quarter of them inside a sample) and return flags."""
+    g = torch.Generator().manual_seed(seed)
+    bins = torch.cumsum(torch.rand((n, S + 1), generator=g) * scale, dim=-1)
+    is_lidar = (torch.arange(n) % 2 == 0)[:, None]
+    dnorm = torch.rand((n, 1), generator=g) * float(bins.max())
+    dnorm[::4] = ((bins[::4, 3] + bins[::4, 4]) * 0.5 + 0.05)[:, None]
+    did_return = torch.rand((n, 1), generator=g) > 0.3
+    return bins, is_lidar, dnorm, did_return
+
+
+def _reference_is_close_to_lidar(bins, is_lidar, dnorm, did_return):
+    """NeuRadarModel._compute_is_close_to_lidar (models/neuradar.py:971-994) on its own RaySamples."""
+    import types
+
+    from nerfstudio.cameras.rays import Frustums, RaySamples
+    from nerfstudio.models.neuradar import NeuRadarModel
+
+    n, S = bins.shape[0], bins.shape[1] - 1
+    md = {"is_lidar": is_lidar[:, None, :].expand(n, S, 1), "directions_norm": dnorm[:, None, :].expand(n, S, 1)}
+    if did_return is not None:
+        md["did_return"] = did_return[:, None, :].expand(n, S, 1)
+    fr = Frustums(origins=torch.zeros((n, S, 3)), directions=torch.zeros((n, S, 3)), starts=bins[:, :-1, None].clone(),
+                  ends=bins[:, 1:, None].clone(), pixel_area=torch.ones((n, S, 1)))
+    rs = RaySamples(frustums=fr, metadata=md)
+    fake_self = types.SimpleNamespace(config=types.SimpleNamespace(loss=types.SimpleNamespace(
+        carving_epsilon=0.1, non_return_lidar_distance=150.0)))
+    NeuRadarModel._compute_is_close_to_lidar(fake_self, rs)
+    return rs.metadata["is_close_to_lidar"][..., 0]
+
+
+def gen_lidar_close():
+    """is_close_to_lidar masks of the carving loss: case a (40 x 16, with and without did_return), case b (64 x 32).
+    Recorded from the reference's own method where the reference modules exist; otherwise from oracle.is_close_to_lidar
+    (which tests/test_oracle_golden.py compares with that method wherever the reference is present).  `source` says
+    which one produced the file (UTF-8 bytes: `bytes(z["source"]).decode()`)."""
+    if HAVE_REFERENCE:
+        close, source = _reference_is_close_to_lidar, "reference: NeuRadarModel._compute_is_close_to_lidar"
+    else:
+        sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+        from oracle import neuradar_oracle as O
+
+        def close(bins, is_lidar, dnorm, did_return):
+            return O.is_close_to_lidar(bins[:, :-1], bins[:, 1:], is_lidar, dnorm, did_return)
+
+        source = "oracle: neuradar_oracle.is_close_to_lidar (reference modules absent)"
+    out = {"source": np.frombuffer(source.encode(), dtype=np.uint8)}
+    for case, (n, S, seed, scale) in {"a": (40, 16, 11, 20.0), "b": (64, 32, 9, 4.0)}.items():
+        bins, is_lidar, dnorm, did_return = _close_inputs(n, S, seed, scale)
+        out.update({f"{case}_bins": bins, f"{case}_is_lidar": is_lidar, f"{case}_dnorm": dnorm, f"{case}_did_return": did_return})
+        out[f"{case}_close"] = close(bins, is_lidar, dnorm, did_return)
+        out[f"{case}_close_no_return"] = close(bins, is_lidar, dnorm, None)
+    save("lidar_close", **out)
+
+
 if __name__ == "__main__":
+    if "--lidar-close-only" in sys.argv:
+        gen_lidar_close()
+        sys.exit(0)
     if "--radar-rays-only" in sys.argv:
         gen_radar_rays()
         sys.exit(0)
@@ -516,3 +576,4 @@ if __name__ == "__main__":
         gen_actors()
         gen_losses()
         gen_radar_rays()
+        gen_lidar_close()

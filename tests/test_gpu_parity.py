@@ -539,6 +539,14 @@ def test_whole_path_with_regularisers_vs_oracle(nb):
     assert report["ok"], report
 
 
+def test_whole_path_under_autocast_vs_oracle(nb):
+    """The step under torch.autocast(float16), as the reference's trainer runs it (engine/trainer.py:564): outputs and
+    every gradient still within the 1e-3 bar of the fp32 oracle."""
+    with torch.autocast("cuda", dtype=torch.float16):
+        report = run_path_parity(num_rays=384, device=DEV, seed=19, train=True)
+    assert report["ok"], report
+
+
 @pytest.mark.parametrize("mode", ["train", "eval"])
 def test_whole_path_golden(nb, golden, mode):
     """The path on the reference's own outputs (tests/golden/path.npz, made by running the reference)."""

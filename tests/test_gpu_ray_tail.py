@@ -107,6 +107,18 @@ def test_carving_vs_reference_model_method():
     assert torch.equal(got.cpu(), want)
 
 
+def test_carving_mask_golden(golden):
+    """The kernel's is_close_to_lidar against the stored masks (tests/golden/lidar_close.npz, gen_lidar_close)."""
+    from neuradar_b200 import functional as Fn
+
+    g = golden("lidar_close")
+    for case in ("a", "b"):
+        bins, is_lidar, dnorm, did_return = (g[f"{case}_{k}"].to(DEV) for k in ("bins", "is_lidar", "dnorm", "did_return"))
+        iv = Fn.SampleIntervals.from_bins(bins)
+        for want, ret in ((g[f"{case}_close"], did_return), (g[f"{case}_close_no_return"], None)):
+            assert torch.equal(Fn.is_close_to_lidar(iv, is_lidar, dnorm, ret).cpu(), want), case
+
+
 def test_nff_outputs_training_extras():
     """get_nff_outputs(calc_lidar_losses=True) emits the training-only outputs of models/neuradar.py:527-546."""
     import neuradar_b200 as nb

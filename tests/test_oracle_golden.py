@@ -295,6 +295,18 @@ def test_is_close_to_lidar_matches_reference_method():
         assert bool(want.any()) and not bool(want.all())
 
 
+def test_is_close_to_lidar_golden(golden):
+    """oracle.is_close_to_lidar against the stored masks (tests/golden/lidar_close.npz, gen_lidar_close), on the inputs of
+    the test above and of tests/test_gpu_ray_tail.py, with and without did_return."""
+    g = golden("lidar_close")
+    for case in ("a", "b"):
+        bins, is_lidar, dnorm, did_return = (g[f"{case}_{k}"] for k in ("bins", "is_lidar", "dnorm", "did_return"))
+        for want, ret in ((g[f"{case}_close"], did_return), (g[f"{case}_close_no_return"], None)):
+            got = O.is_close_to_lidar(bins[:, :-1], bins[:, 1:], is_lidar, dnorm, ret)
+            assert torch.equal(got, want), case
+            assert bool(want.any()) and not bool(want.all())
+
+
 def test_radar_rays(golden):
     """Radar ray generation (SURVEY.md 8f next-4) against Radars._generate_rays_from_fov of the reference."""
     g = golden("radar_rays")
