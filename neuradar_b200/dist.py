@@ -21,6 +21,8 @@ import torch
 import torch.distributed as dist
 from torch import Tensor, nn
 
+from ._lib import NeuradarB200Error
+
 
 def shard_bounds(num_rays: int, world_size: int, rank: int, granule: int = 1) -> Tuple[int, int]:
     """Contiguous slice [start, end) of a global ray batch owned by `rank`.
@@ -36,10 +38,10 @@ def shard_bounds(num_rays: int, world_size: int, rank: int, granule: int = 1) ->
     return start * granule, end * granule
 
 
-def _world(group=None) -> int:
+def _world() -> int:
     if not dist.is_available() or not dist.is_initialized():
         return 1
-    return dist.get_world_size(group)
+    return dist.get_world_size()
 
 
 class PeerMemory:
@@ -47,13 +49,12 @@ class PeerMemory:
     flag area, for `nrb_peer_all_reduce` (csrc/peer_reduce.cu).  Built on torch.distributed._symmetric_memory, which only
     provides the mapping; the collective is this package's kernel."""
 
-    def __init__(self, numel: int, device, group=None):
+    def __init__(self, numel: int, device):
         import ctypes as C
 
         import torch.distributed._symmetric_memory as symm
 
-        self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
-        pg = group if group is not None else dist.group.WORLD
+        self.world, self.rank, pg = dist.get_world_size(), dist.get_rank(), dist.group.WORLD
         self.flat = symm.empty(numel, dtype=torch.float32, device=device)
         self.flags = symm.empty(256, dtype=torch.int32, device=device)  # 4 slots x 64 words (peer_reduce.cu: kSlotWords)
         self.flat.zero_()
@@ -74,7 +75,7 @@ class PeerMemory:
         self.buffer_ptrs = (C.c_uint64 * self.world)(*bufs)
         self.flag_ptrs = (C.c_uint64 * self.world)(*sigs)
         torch.cuda.synchronize(device)
-        dist.barrier(group)  # every rank's flags are zero before anyone's first collective
+        dist.barrier()  # every rank's flags are zero before anyone's first collective
 
     def all_reduce(self, slot: int, offset: int, n: int, scale: float, max_ctas: int = 0) -> None:
         """In place over floats [offset, offset + n) of every rank's buffer, on the current stream."""
@@ -84,25 +85,29 @@ class PeerMemory:
                   n, float(scale), max_ctas, _lib.stream_ptr())
 
 
-def peer_memory_or_none(numel: int, device, group=None) -> Optional[PeerMemory]:
+def peer_memory_or_none(numel: int, device) -> Optional[PeerMemory]:
     """Symmetric memory for the arena when this is a single-box NCCL job of at most 8 ranks (NRB_PEER_REDUCE=0 disables)."""
-    if os.environ.get("NRB_PEER_REDUCE", "1") == "0" or _world(group) == 1 or torch.device(device).type != "cuda":
-        return None
-    if dist.get_backend(group) != "nccl" or dist.get_world_size(group) > 8 or group is not None:
+    if (os.environ.get("NRB_PEER_REDUCE", "1") == "0" or _world() == 1 or torch.device(device).type != "cuda"
+            or dist.get_backend() != "nccl" or dist.get_world_size() > 8):
         return None
     if int(os.environ.get("LOCAL_WORLD_SIZE", dist.get_world_size())) != dist.get_world_size():
         return None  # more than one box: the ranks do not share an NVSwitch domain
     pm = None
     try:
-        pm = PeerMemory(numel, device, group)
+        pm = PeerMemory(numel, device)
     except Exception as e:  # noqa: BLE001 - no peer mapping on this system: NCCL carries the collective
         import warnings
 
         warnings.warn(f"neuradar_b200: peer-memory all-reduce unavailable ({type(e).__name__}: {str(e)[:120]}); using NCCL")
     # every rank must take the same route: agree on the outcome
     ok = torch.tensor([1 if pm is not None else 0], device=device, dtype=torch.int32)
-    dist.all_reduce(ok, op=dist.ReduceOp.MIN, group=group)
+    dist.all_reduce(ok, op=dist.ReduceOp.MIN)
     return pm if int(ok.item()) == 1 else None
+
+
+def padded_numel(n: int) -> int:
+    """Floats a view of `n` elements takes in a flat gradient buffer: 16-byte aligned for the scatters' vector atomics."""
+    return (n + 3) // 4 * 4
 
 
 class OverlappedReduce:
@@ -110,34 +115,40 @@ class OverlappedReduce:
 
     `start_early()` (called by the backward of the kernel that produced those gradients, on the stream it ran on) launches
     their all-reduce on a side stream; `finish()` reduces the rest and joins.  Without an early call `finish()` reduces
-    everything in one collective.  Single process: no-ops."""
+    everything in one collective.  Single process: no-ops.  States: idle -> (start_early) in flight -> (finish) idle; a
+    second `start_early()` in flight raises, as the write that caused it would never be exchanged.  The constructor is a
+    collective point: it creates the side stream and the early piece's communicator, so the backward creates nothing."""
 
     def __init__(self, flat: Tensor, n_early: int = 0, peer: Optional[PeerMemory] = None):
         self.flat, self.n_early = flat, int(n_early)
-        self.peer = peer  # the arena lives in symmetric memory: this package's NVLink kernel instead of NCCL
-        self._work = None
-        self._stream: Optional[torch.cuda.Stream] = None
-        self.group = None
-        self._early = None
+        self.peer = peer  # the buffer lives in symmetric memory: this package's NVLink kernel instead of NCCL
+        self._work = None  # idle; in flight: the early collective (True on the peer-memory route)
+        overlap = self.n_early > 0 and _world() > 1 and flat.is_cuda
+        self._stream = torch.cuda.Stream(device=flat.device) if overlap else None
+        self._early_group = self._cta_limited_group() if overlap and peer is None else None  # None: the default one
 
     early_ctas = int(os.environ.get("NRB_EARLY_REDUCE_CTAS", "8"))
     """CTAs NCCL may use for the EARLY collective.  It runs beside the proposal backward, which it slows down in proportion
     to the SMs it occupies (B200 x8, 64 MiB: 16+ CTAs by default, 0.28 ms alone, +0.15 ms on the overlapped kernels;
     8 CTAs: 0.50 ms alone, still well inside the 1.3 ms it has to hide in; profiles/r2_nccl_probe_n8.txt)."""
 
-    def _early_group(self):
-        """A second NCCL communicator over the same ranks whose kernels are limited to `early_ctas` CTAs."""
-        if self._early is None:
-            self._early = self.group
-            if self.early_ctas > 0 and self.flat.is_cuda and dist.get_backend(self.group) == "nccl" and self.group is None:
-                try:
-                    opts = dist.ProcessGroupNCCL.Options()
-                    opts.config.max_ctas = self.early_ctas
-                    opts.config.min_ctas = 1
-                    self._early = dist.new_group(backend="nccl", pg_options=opts)
-                except Exception:  # noqa: BLE001 - an older torch / NCCL without communicator configs: use the default one
-                    self._early = self.group
-        return self._early
+    def _cta_limited_group(self):
+        """A second NCCL communicator over the same ranks whose kernels are limited to `early_ctas` CTAs (None: default)."""
+        if self.early_ctas <= 0 or dist.get_backend() != "nccl":
+            return None
+        try:
+            opts = dist.ProcessGroupNCCL.Options()
+            opts.config.max_ctas = self.early_ctas
+            opts.config.min_ctas = 1
+            return dist.new_group(backend="nccl", pg_options=opts)
+        except Exception:  # noqa: BLE001 - an older torch / NCCL without communicator configs: use the default one
+            return None
+
+    def use_nccl(self) -> None:
+        """Reduce with NCCL although the buffer is in symmetric memory.  A collective point, like the constructor."""
+        self.peer = None
+        if self._stream is not None:
+            self._early_group = self._cta_limited_group()
 
     peer_ctas = int(os.environ.get("NRB_PEER_CTAS", "0"))
     """CTAs of the peer-memory kernel (0 = measured defaults, profiles/r2_peer_reduce_probe.txt): with in-switch reduction
@@ -152,47 +163,42 @@ class OverlappedReduce:
         return 16 if early else 0
 
     def start_early(self) -> None:
-        if self.n_early <= 0 or self._work is not None or _world(self.group) == 1:
+        if self.n_early <= 0 or _world() == 1:
             return
-        if self.flat.is_cuda:
-            if self._stream is None:
-                self._stream = torch.cuda.Stream(device=self.flat.device)
-            self._stream.wait_stream(torch.cuda.current_stream(self.flat.device))
-            if self.peer is not None:
-                with torch.cuda.stream(self._stream):  # (already averaged: finish() returns 1)
-                    self.peer.all_reduce(0, 0, self.n_early, 1.0 / self.peer.world, self._peer_ctas(True))
+        if self._work is not None:
+            raise NeuradarB200Error("early gradients written again while their all-reduce was in flight: under data "
+                                    "parallelism one backward per all_reduce() (no gradient accumulation, no second backward)")
+        if not self.flat.is_cuda:
+            self._work = dist.all_reduce(self.flat[: self.n_early], op=dist.ReduceOp.SUM, async_op=True)
+            return
+        self._stream.wait_stream(torch.cuda.current_stream(self.flat.device))
+        with torch.cuda.stream(self._stream):
+            if self.peer is not None:  # (already averaged: finish() returns 1)
+                self.peer.all_reduce(0, 0, self.n_early, 1.0 / self.peer.world, self._peer_ctas(True))
                 self._work = True
-                return
-            group = self._early_group()
-            with torch.cuda.stream(self._stream):
-                self._work = dist.all_reduce(self.flat[: self.n_early], op=dist.ReduceOp.SUM, group=group, async_op=True)
-        else:
-            self._work = dist.all_reduce(self.flat[: self.n_early], op=dist.ReduceOp.SUM, group=self.group, async_op=True)
+            else:
+                self._work = dist.all_reduce(self.flat[: self.n_early], op=dist.ReduceOp.SUM, group=self._early_group,
+                                             async_op=True)
 
     def finish(self, group=None) -> float:
         """Sum over ranks; returns the factor that still has to be applied for the average: 1 / world_size after NCCL (the
         caller applies it or hands it to the optimiser), 1 after the peer-memory kernel (which averages in place)."""
-        world = _world(group)
+        if group is not None and group is not dist.group.WORLD:
+            raise ValueError("only the default process group is supported")
+        world = _world()
         if world == 1:
             return 1.0
+        early, self._work = self._work, None
+        lo = self.n_early if early is not None else 0
         if self.peer is not None:  # sums AND averages in place (the x 1/world rides in the kernel)
-            total = self.flat.numel()
-            if self._work is not None:
-                self.peer.all_reduce(1, self.n_early, total - self.n_early, 1.0 / world, self._peer_ctas(False))
-                torch.cuda.current_stream(self.flat.device).wait_stream(self._stream)
-                self._work = None
-            else:
-                self.peer.all_reduce(1, 0, total, 1.0 / world, self._peer_ctas(False))
-            return 1.0
-        if self._work is not None:
-            dist.all_reduce(self.flat[self.n_early :], op=dist.ReduceOp.SUM, group=group)
-            self._work.wait()  # the current stream waits for the early collective
-            if self._stream is not None:
-                torch.cuda.current_stream(self.flat.device).wait_stream(self._stream)
-            self._work = None
+            self.peer.all_reduce(1, lo, self.flat.numel() - lo, 1.0 / world, self._peer_ctas(False))
         else:
-            dist.all_reduce(self.flat, op=dist.ReduceOp.SUM, group=group)
-        return 1.0 / world
+            dist.all_reduce(self.flat[lo:], op=dist.ReduceOp.SUM)
+            if early is not None:
+                early.wait()  # the current stream waits for the early collective
+        if early is not None and self._stream is not None:
+            torch.cuda.current_stream(self.flat.device).wait_stream(self._stream)
+        return 1.0 if self.peer is not None else 1.0 / world
 
 
 def order_early_first(params: Sequence[nn.Parameter], early: Optional[Iterable[nn.Parameter]]) -> Tuple[List[nn.Parameter], int]:
@@ -208,13 +214,15 @@ class GradArena:
     `param.grad` is pointed into the arena, so autograd accumulates straight into it, `zero()` is one memset and
     `all_reduce()` is one or two collectives (see OverlappedReduce).  Parameters that receive no gradient in a step
     (e.g. the never-evaluated first proposal field) simply contribute zeros, which is what DDP's find_unused_parameters
-    does.  `direct_scatter=True` additionally lets the hash-grid backward kernels add straight into the arena
-    (functional.grad_sink_of) instead of returning a table-sized temporary to autograd.  `early` names the parameters
-    (hash tables with a direct sink) whose gradient is complete when their backward kernel has run.
+    does.  `direct_scatter=True` additionally lets the backward kernels add straight into the arena
+    (`param._nrb_grad_sink`, functional.grad_sink_of) instead of returning a temporary to autograd.  `early` names the
+    parameters (hash tables with a direct sink) whose gradient is complete when their backward kernel has run; they lead
+    the buffer and that kernel's backward starts their reduction (`param._nrb_grad_ready`).  A gradient a parameter
+    already has when the arena is built is copied into its view.
 
     Contract: gradients must stay views of the arena.  `optimizer.zero_grad()` / `module.zero_grad()` default to
-    set_to_none=True and would detach them; `zero()` and `all_reduce()` therefore re-link (`relink()`): a gradient that
-    was replaced is copied back into its view, one that was set to None is treated as zero."""
+    set_to_none=True and would detach them; `zero()` and `all_reduce()` therefore re-link (`relink()`).  Under data
+    parallelism with `early`, exactly one backward runs per `all_reduce()`, and every rank runs it."""
 
     def __init__(self, params: Iterable[nn.Parameter], skip_unused: Optional[List[nn.Parameter]] = None,
                  direct_scatter: bool = False, early: Optional[Iterable[nn.Parameter]] = None):
@@ -223,25 +231,22 @@ class GradArena:
         if not params:
             raise ValueError("no trainable parameters")
         self.params, n_first = order_early_first(params, early if direct_scatter else None)
-        dev, total = self.params[0].device, 0
-        self.offsets = []
-        n_early = 0
-        for i, p in enumerate(self.params):
-            if p.dtype != torch.float32 or p.device != dev:
-                raise ValueError("GradArena expects fp32 parameters on one device")
-            self.offsets.append(total)
-            total += (p.numel() + 3) // 4 * 4  # keep every view 16-byte aligned for the vector atomics
-            if i < n_first:
-                n_early = total
-        self.peer = peer_memory_or_none(total, dev)
-        self.flat = self.peer.flat if self.peer is not None else torch.zeros((total,), device=dev, dtype=torch.float32)
-        self.direct_scatter = direct_scatter
-        self.reducer = OverlappedReduce(self.flat, n_early, self.peer)
+        dev = self.params[0].device
+        if any(p.dtype != torch.float32 or p.device != dev for p in self.params):
+            raise ValueError("GradArena expects fp32 parameters on one device")
+        sizes = [padded_numel(p.numel()) for p in self.params]
+        self.offsets = [sum(sizes[:i]) for i in range(len(sizes))]
+        total, n_early = sum(sizes), sum(sizes[:n_first])
+        peer = peer_memory_or_none(total, dev)
+        self.flat = peer.flat if peer is not None else torch.zeros((total,), device=dev, dtype=torch.float32)
+        self.reducer = OverlappedReduce(self.flat, n_early, peer)
         self._views = [self.flat[off : off + p.numel()].view_as(p) for p, off in zip(self.params, self.offsets)]
         for i, (p, view) in enumerate(zip(self.params, self._views)):
+            if p.grad is not None:
+                view.copy_(p.grad)
             p.grad = view
             if direct_scatter:
-                p._nrb_grad_sink = view  # the backward kernels add straight into the arena (functional.grad_sink_of)
+                p._nrb_grad_sink = view
                 if i < n_first:
                     p._nrb_grad_ready = self.reducer.start_early
 
@@ -249,16 +254,25 @@ class GradArena:
     def nbytes(self) -> int:
         return self.flat.numel() * 4
 
+    @property
+    def peer(self) -> Optional[PeerMemory]:  # None: NCCL (or a single process)
+        return self.reducer.peer
+
     def relink(self) -> int:
-        """Point every `param.grad` back into the arena; returns how many had been detached."""
+        """Point every `param.grad` back into the arena; returns how many had been detached.  A gradient that was replaced
+        is copied into its view.  One that was set to None counts as zero, unless the parameter has a sink: the backward
+        kernels add into the sink whatever `.grad` is, so its view already holds the gradient."""
         fixed = 0
         for p, view in zip(self.params, self._views):
             if p.grad is not None and p.grad.data_ptr() == view.data_ptr():
                 continue
+            sink = getattr(p, "_nrb_grad_sink", None) is not None
             if p.grad is not None:
                 view.copy_(p.grad)
+            elif not sink:
+                view.zero_()
             p.grad = view
-            if getattr(p, "_nrb_grad_sink", None) is not None:
+            if sink:
                 p._nrb_grad_sink = view
             fixed += 1
         return fixed
@@ -269,10 +283,14 @@ class GradArena:
             if p.grad is None or p.grad.data_ptr() != view.data_ptr():
                 p.grad = view
 
-    def all_reduce(self, group=None, average: bool = True) -> None:
+    def reduce(self, group=None) -> float:
+        """Re-link, then sum over the ranks of the default process group; returns the factor that makes it the average."""
         self.relink()
-        mult = self.reducer.finish(group)
+        return self.reducer.finish(group)
+
+    def all_reduce(self, group=None, average: bool = True) -> None:
+        mult = self.reduce(group)
         if average and mult != 1.0:
             self.flat.mul_(mult)
-        elif not average and self.peer is not None and _world(group) > 1:
-            self.flat.mul_(float(_world(group)))  # (the peer-memory kernel averages in place)
+        elif not average and self.peer is not None and _world() > 1:
+            self.flat.mul_(float(_world()))  # (the peer-memory kernel averages in place)

@@ -6,7 +6,8 @@ Shapes follow the reference: N rays, S samples per ray, M = N*S points, L levels
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
+from types import SimpleNamespace
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -15,6 +16,7 @@ from torch.amp import custom_bwd, custom_fwd
 
 from . import _lib
 from ._lib import Grid, Intervals, Mlp, MlpGrad, Rays, Spacing, check, f32c, ptr, stream_ptr
+from .dist import padded_numel
 
 
 # ------------------------------------------------------------------------------------------------
@@ -191,36 +193,82 @@ def note_consumer_stream(device) -> None:
     _CONSUMER_STREAMS[device] = torch.cuda.current_stream(device)
 
 
-def _sink_written(table: Tensor) -> None:
-    """Called by a backward that added straight into a gradient sink (no tensor is returned to autograd for it, so
-    autograd's own stream bookkeeping does not cover the write).  (1) If the backward ran on a side stream - autograd
-    replays a node on the stream its forward ran on - the default stream is made to wait for it, so that an all-reduce
-    or optimiser step issued after `loss.backward()` cannot race with the scatter.  (2) The owner of the sink may have
-    registered a callback (dist.OverlappedReduce.start_early) to start reducing this gradient right away."""
-    dev = table.device
+def _sink_written(params: Sequence[Tensor]) -> None:
+    """Called once by a backward that added straight into the gradient sinks of `params` (no tensor is returned to
+    autograd for them, so autograd's own stream bookkeeping does not cover the writes).  (1) If the backward ran on a
+    side stream - autograd replays a node on the stream its forward ran on - the default stream is made to wait for it,
+    so that an all-reduce or optimiser step issued after `loss.backward()` cannot race with the scatter.  (2) The owner of
+    a sink may have registered a callback (dist.OverlappedReduce.start_early) to start reducing that gradient right away."""
+    dev = params[0].device
     cur = torch.cuda.current_stream(dev)
     if not torch.cuda.is_current_stream_capturing():  # (a graph capture orders its own streams)
         # the default stream and the stream the forward was issued from (`note_consumer_stream`): whoever reads the sink next
-        waiters = {torch.cuda.default_stream(dev)}
-        consumer = _CONSUMER_STREAMS.get(dev)
-        if consumer is not None:
-            waiters.add(consumer)
-        waiters.discard(cur)
+        waiters = {torch.cuda.default_stream(dev), _CONSUMER_STREAMS.get(dev, cur)} - {cur}
         if waiters:
-            ev = torch.cuda.Event()
-            ev.record(cur)
+            ev = cur.record_event()
             for s in waiters:
                 s.wait_event(ev)
-    ready = getattr(table, "_nrb_grad_ready", None)
-    if ready is not None:
-        ready()
+    for p in params:
+        ready = getattr(p, "_nrb_grad_ready", None)
+        if ready is not None:
+            ready()
+
+
+class _GradSinks:
+    """The gradient sinks (`grad_sink_of`) of an autograd node's parameters, looked up by its forward.  The backward takes
+    each gradient buffer from `dest()` / `packed_dests()` (the sink, or zeroed memory whose content goes back to autograd),
+    launches, and returns what `written()` gives back."""
+
+    def __init__(self, params: Sequence[Optional[Tensor]]):
+        self.params = list(params)
+        self.sinks = [grad_sink_of(p) for p in self.params]
+
+    def dest(self, i: int) -> Tensor:
+        p = self.params[i]
+        return self.sinks[i] if self.sinks[i] is not None else torch.zeros(p.shape, device=p.device, dtype=torch.float32)
+
+    def packed_dests(self, idx: range) -> List[Optional[Tensor]]:
+        """`dest()` of the parameters `idx` (None for a None parameter), with the zeroed ones packed into ONE scratch
+        buffer: one memset instead of one per parameter."""
+        need = [self.params[i] for i in idx if self.params[i] is not None and self.sinks[i] is None]
+        scratch = torch.zeros((sum(padded_numel(p.numel()) for p in need),), device=need[0].device,
+                              dtype=torch.float32) if need else None
+        out, off = [], 0
+        for i in idx:
+            p, sink = self.params[i], self.sinks[i]
+            if p is None or sink is not None:
+                out.append(sink)
+            else:
+                out.append(scratch[off : off + p.numel()].view(p.shape))
+                off += padded_numel(p.numel())
+        return out
+
+    def written(self, grads: Sequence[Optional[Tensor]]) -> List[Optional[Tensor]]:
+        """Called once after the launches with one buffer per parameter: orders and signals every sink (`_sink_written`);
+        returns `grads` with None where a sink took the gradient."""
+        written = [p for p, sink in zip(self.params, self.sinks) if sink is not None]
+        if written:
+            _sink_written(written)
+        return [None if sink is not None else g for g, sink in zip(grads, self.sinks)]
+
+
+def _save(ctx, **named) -> None:
+    """ctx.save_for_backward, once, under names; a value is a tensor, None or a list of them.  `_saved(ctx)` gives them
+    back as attributes."""
+    ctx.saved_layout = [(k, len(v) if isinstance(v, list) else -1) for k, v in named.items()]
+    ctx.save_for_backward(*[t for v in named.values() for t in (v if isinstance(v, list) else [v])])
+
+
+def _saved(ctx) -> SimpleNamespace:
+    it = iter(ctx.saved_tensors)
+    return SimpleNamespace(**{k: next(it) if n < 0 else [next(it) for _ in range(n)] for k, n in ctx.saved_layout})
 
 
 class _HashEncode(torch.autograd.Function):
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
     def forward(ctx, x, table, std, spec: GridSpec, samples_per_ray: int = 0):
-        ctx.sink = grad_sink_of(table)
+        ctx.sinks = _GradSinks([table])
         x = f32c(x)
         table = f32c(table)
         std = None if std is None else f32c(std.reshape(-1))
@@ -240,15 +288,13 @@ class _HashEncode(torch.autograd.Function):
         spec = ctx.spec
         dy = f32c(dy)
         need_dx = ctx.needs_input_grad[0]
-        dtable = ctx.sink if ctx.sink is not None else torch.zeros_like(table)
+        dtable = ctx.sinks.dest(0)
         dx = torch.empty_like(x) if need_dx else None
         g = spec.struct(table)
         ws, ws_bytes = _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(g), x.shape[0])), x.device)
         _lib.call("nrb_hash_bwd", C.byref(g), ptr(x), ptr(std), ptr(dy), ptr(dtable), ptr(dx), x.shape[0], ws, ws_bytes,
                   stream_ptr(), tag="nrb_hash_bwd:" + spec.tag)
-        if ctx.sink is not None:
-            _sink_written(table)
-        return dx, (None if ctx.sink is not None else dtable), None, None, None
+        return dx, *ctx.sinks.written([dtable]), None, None, None
 
 
 def hash_encode(x: Tensor, table: Tensor, spec: GridSpec, std: Optional[Tensor] = None, samples_per_ray: int = 0) -> Tensor:
@@ -312,20 +358,15 @@ class _MlpForward(torch.autograd.Function):
         hidden = torch.empty((n_hidden, M), device=x.device, dtype=torch.float32) if keep else None
         m = _mlp_struct(dims, weights, biases)
         _lib.call("nrb_mlp_fwd", C.byref(m), ptr(x), ptr(y), ptr(hidden), M, stream_ptr(), tag="nrb_mlp_fwd:" + "x".join(map(str, dims)))
-        ctx.save_for_backward(x, hidden, *weights, *[b for b in biases if b is not None])
-        ctx.has_bias = [b is not None for b in biases]
+        _save(ctx, x=x, hidden=hidden, weights=weights, biases=biases)
         ctx.dims = dims
         return y
 
     @staticmethod
     @custom_bwd(device_type="cuda")
     def backward(ctx, dy):
-        saved = ctx.saved_tensors
-        x, hidden = saved[0], saved[1]
-        n = len(ctx.dims) - 1
-        weights = list(saved[2 : 2 + n])
-        rest = list(saved[2 + n :])
-        biases = [rest.pop(0) if hb else None for hb in ctx.has_bias]
+        s = _saved(ctx)
+        x, hidden, weights, biases, n = s.x, s.hidden, s.weights, s.biases, len(ctx.dims) - 1
         dy = f32c(dy)
         M = x.shape[0]
         dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
@@ -381,9 +422,9 @@ class ActorBatch:
     tables: List[Tensor]
     spec: GridSpec  # of ONE actor grid
 
-    def grids_struct(self, tables: Optional[Sequence[Tensor]] = None) -> "_lib.ActorGrids":
+    def grids_struct(self) -> "_lib.ActorGrids":
         g = _lib.ActorGrids()
-        for i, t in enumerate(tables if tables is not None else self.tables):
+        for i, t in enumerate(self.tables):
             g.tables[i] = ptr(t)
         for i, sc in enumerate(self.spec.scalings):
             g.scalings[i] = sc
@@ -395,6 +436,16 @@ class ActorBatch:
         a = _lib.ActorSamples()
         a.grid_id, a.pos, a.std, a.dirs = ptr(self.grid_id), ptr(self.pos), ptr(self.std), ptr(self.dirs)
         return a
+
+    def with_tables(self, tables: Sequence[Tensor]) -> "ActorBatch":
+        return replace(self, tables=list(tables))
+
+    def to_save(self) -> List[Tensor]:  # what `from_saved` rebuilds the batch from
+        return [self.grid_id, self.pos, self.std, self.dirs, *self.tables]
+
+    @classmethod
+    def from_saved(cls, saved: Sequence[Tensor], spec: GridSpec) -> "ActorBatch":
+        return cls(*saved[:4], list(saved[4:]), spec)
 
 
 def actor_assign(rays: RayData, iv: SampleIntervals, world2boxes: Tensor, valid: Tensor, bounds: Tensor, actor_to_id: Tensor,
@@ -421,38 +472,21 @@ def actor_assign(rays: RayData, iv: SampleIntervals, world2boxes: Tensor, valid:
 # ------------------------------------------------------------------------------------------------
 # fused field: hash gather + both MLPs in one kernel; backward recomputes the activations
 # ------------------------------------------------------------------------------------------------
-def _field_fused_backward(ctx, saved_tensors, dfeature, dfeat_ray, weights, dsdf, dalpha):
-    """Shared by the two autograd Functions that end in the fused field kernel.  Returns (dx or None, dbeta, dws, dbs);
-    in gather mode the hash-table gradient is scattered here (into the direct sink or a fresh tensor kept on ctx)."""
-    table, x3, std, ximg, masks, sh, beta, sdf, alpha = saved_tensors[:9]
-    weights_ = list(saved_tensors[9:14])
-    rest = list(saved_tensors[14:])
-    biases = [rest.pop(0) if hb else None for hb in ctx.has_bias]
-    actors = None
-    if ctx.actor_spec is not None:  # [grid_id, pos, std, dirs, *tables] ride at the end
-        actors = ActorBatch(rest[0], rest[1], rest[2], rest[3], list(rest[4:]), ctx.actor_spec)
-    M, dev = sdf.shape[0], sdf.device
+def _field_fused_backward(ctx, s: SimpleNamespace, dfeature, dfeat_ray, weights, dsdf, dalpha):
+    """Shared by the two autograd Functions that end in the fused field kernel; `s` is `_saved(ctx)`.  Returns (dx or None,
+    the gradients of [table, beta, w0..w4, b0..b4, *actor tables] for autograd); in gather mode the hash-table gradient
+    is scattered here too."""
+    actors = None if ctx.actor_spec is None else ActorBatch.from_saved(s.actors, ctx.actor_spec)
+    M, dev = s.sdf.shape[0], s.sdf.device
     need_dx = ctx.gather or ctx.needs_x_grad
     dximg = torch.empty((int(_lib_().nrb_field_fused_image_bytes(M)) // 4,), device=dev, dtype=torch.float32) if need_dx else None
-    # parameter gradients: straight into the owner's flat buffer where a sink was registered, else one zeroed scratch
-    psinks = ctx.param_sinks  # [beta, w0..w4, b0..b4] (None = no sink)
-    tensors = [beta, *weights_, *biases]
-    need = [t for t, sk in zip(tensors, psinks) if t is not None and sk is None]
-    scratch = torch.zeros((sum((t.numel() + 3) // 4 * 4 for t in need),), device=dev, dtype=torch.float32) if need else None
-    grads, off = [], 0
-    for t, sk in zip(tensors, psinks):
-        if t is None:
-            grads.append(None)
-        elif sk is not None:
-            grads.append(sk)
-        else:
-            grads.append(scratch[off : off + t.numel()].view_as(t))
-            off += (t.numel() + 3) // 4 * 4
-    dbeta_t, dws, dbs = grads[0], grads[1:6], grads[6:11]
-    m = _field_struct(weights_, biases, beta, ctx.beta_min)
+    sinks = ctx.sinks  # [table, beta, w0..w4, b0..b4, *actor tables]
+    dmlp = sinks.packed_dests(range(1, 12))
+    dbeta, dws, dbs = dmlp[0], dmlp[1:6], dmlp[6:11]
+    m = _field_struct(s.weights, s.biases, s.beta, ctx.beta_min)
     bi = _lib.FieldFusedBwdIn()
-    bi.saved.ximg, bi.saved.masks, bi.saved.ld = ptr(ximg), ptr(masks), masks.shape[1]
-    bi.sh, bi.sdf, bi.alpha = ptr(sh), ptr(sdf), ptr(alpha)
+    bi.saved.ximg, bi.saved.masks, bi.saved.ld = ptr(s.ximg), ptr(s.masks), s.masks.shape[1]
+    bi.sh, bi.sdf, bi.alpha = ptr(s.sh), ptr(s.sdf), ptr(s.alpha)
     bi.dfeature, bi.dfeat_ray, bi.weights = ptr(dfeature), ptr(dfeat_ray), ptr(weights)
     bi.dsdf, bi.dalpha = ptr(dsdf), ptr(dalpha)
     if actors is not None:
@@ -462,45 +496,39 @@ def _field_fused_backward(ctx, saved_tensors, dfeature, dfeat_ray, weights, dsdf
     for i in range(5):
         bo.dweights[i] = ptr(dws[i])
         bo.dbiases[i] = ptr(dbs[i])
-    bo.dbeta = ptr(dbeta_t)
+    bo.dbeta = ptr(dbeta)
     _lib.call("nrb_field_fused_bwd", C.byref(m), C.byref(bi), C.byref(bo), ctx.samples_per_ray, M, stream_ptr())
     dx = dtable = None
     if ctx.gather:
         spec = ctx.spec
-        dtable = ctx.sink if ctx.sink is not None else torch.zeros_like(table)
-        g = spec.struct(table)
+        dtable = sinks.dest(0)
+        g = spec.struct(s.table)
         ws, ws_bytes = _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(g), M)), dev)
-        _lib.call("nrb_hash_bwd_image", C.byref(g), ptr(x3), ptr(std), ptr(dximg), ptr(dtable),
+        _lib.call("nrb_hash_bwd_image", C.byref(g), ptr(s.x3), ptr(s.std), ptr(dximg), ptr(dtable),
                   None if actors is None else ptr(actors.grid_id), M, ws, ws_bytes, stream_ptr(), tag="nrb_hash_bwd:" + spec.tag)
-        if ctx.sink is not None:
-            _sink_written(table)
-            dtable = None
     elif ctx.needs_x_grad:
         dx = dximg.view(-1, 8, 128, 4).permute(0, 2, 1, 3).reshape(-1, 32)[:M]
     dactor = []
     if actors is not None:  # the actor samples' gradient goes to their own tables
-        dactor = [sk if sk is not None else torch.zeros_like(t) for t, sk in zip(actors.tables, ctx.actor_sinks)]
+        dactor = [sinks.dest(i) for i in range(12, len(sinks.params))]
         arr = (C.c_void_p * len(dactor))(*[ptr(t) for t in dactor])
         ag, asmp = actors.grids_struct(), actors.samples_struct()
         _lib.call("nrb_actor_scatter", C.byref(ag), arr, C.byref(asmp), ptr(dximg), None, M, stream_ptr())
-        dactor = [None if sk is not None else t for t, sk in zip(dactor, ctx.actor_sinks)]
-    ctx.dactor = dactor
-    if any(sk is not None for sk in psinks):
-        _sink_written(next(t for t, sk in zip(tensors, psinks) if sk is not None))
-    ret = [None if sk is not None else gr for gr, sk in zip(grads, psinks)]
-    return dx, dtable, ret[0], ret[1:6], ret[6:11]
+    return dx, sinks.written([dtable, *dmlp, *dactor])
 
 
-def _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, spec, beta, params, train, param_sinks=None,
+def _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, spec, beta, params, train,
                          actors: Optional[ActorBatch] = None):
-    """Launch nrb_field_fused_fwd and stash what the backward needs on ctx.  Returns (feature, sdf, alpha)."""
+    """Launch nrb_field_fused_fwd and set on ctx what the backward needs besides tensors.  Returns (feature, sdf, alpha,
+    the tensors to save by name or None when not training)."""
     gather = table is not None
+    ctx.sinks = _GradSinks([table, beta, *params])
     sh, beta = f32c(sh.detach()), f32c(beta)
     weights = [f32c(w) for w in params[:5]]
     biases = [None if b is None else f32c(b) for b in params[5:10]]
     ag = asmp = None
     if actors is not None:
-        actors = ActorBatch(actors.grid_id, actors.pos, actors.std, actors.dirs, [f32c(t) for t in params[10:]], actors.spec)
+        actors = actors.with_tables([f32c(t) for t in params[10:]])
         ag, asmp = actors.grids_struct(), actors.samples_struct()
     if gather:
         table, x3 = f32c(table), f32c(x3)
@@ -524,17 +552,12 @@ def _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, 
               ptr(std) if gather else None, None if gather else ptr(x), ptr(sh), int(samples_per_ray), M, ptr(feature),
               ptr(sdf), ptr(alpha), C.byref(sv), None if ag is None else C.byref(ag), None if asmp is None else C.byref(asmp),
               stream_ptr())
-    ctx.actor_spec = None
-    if train:
-        extra = [] if actors is None else [actors.grid_id, actors.pos, actors.std, actors.dirs, *actors.tables]
-        ctx.actor_spec = None if actors is None else actors.spec
-        ctx.actor_sinks = [] if actors is None else [grad_sink_of(t) for t in params[10:]]
-        ctx.save_for_backward(table if gather else None, x3 if gather else None, std if gather else None, ximg, masks, sh,
-                              beta, sdf, alpha, *weights, *[b for b in biases if b is not None], *extra)
-        ctx.has_bias = [b is not None for b in biases]
-        ctx.samples_per_ray, ctx.beta_min, ctx.gather, ctx.spec = int(samples_per_ray), float(beta_min), gather, spec
-        ctx.param_sinks = param_sinks if param_sinks is not None else [None] * 11
-    return feature, sdf, alpha
+    ctx.actor_spec = None if actors is None else actors.spec
+    ctx.samples_per_ray, ctx.beta_min, ctx.gather, ctx.spec = int(samples_per_ray), float(beta_min), gather, spec
+    saved = None if not train else dict(
+        table=table if gather else None, x3=x3 if gather else None, std=std if gather else None, ximg=ximg, masks=masks,
+        sh=sh, beta=beta, sdf=sdf, alpha=alpha, weights=weights, biases=biases, actors=[] if actors is None else actors.to_save())
+    return feature, sdf, alpha, saved
 
 
 class _FieldFused(torch.autograd.Function):
@@ -544,23 +567,23 @@ class _FieldFused(torch.autograd.Function):
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
     def forward(ctx, table, x, x3, std, sh, samples_per_ray: int, beta_min: float, spec, actors, beta, *params):
-        ctx.sink = grad_sink_of(table) if table is not None else None
         train = any(ctx.needs_input_grad)
         ctx.needs_x_grad = x is not None and ctx.needs_input_grad[1]
-        sinks = [grad_sink_of(beta)] + [grad_sink_of(q) for q in params[:10]]
-        return _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, spec, beta, params, train, sinks,
-                                    actors)
+        feature, sdf, alpha, saved = _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, spec, beta,
+                                                          params, train, actors)
+        if train:
+            _save(ctx, **saved)
+        return feature, sdf, alpha
 
     @staticmethod
     @custom_bwd(device_type="cuda")
     def backward(ctx, dfeature, dsdf, dalpha):
-        M = ctx.saved_tensors[7].shape[0]
-        dev = ctx.saved_tensors[7].device
-        dfeature = torch.zeros((M, 32), device=dev) if dfeature is None else f32c(dfeature)
+        s = _saved(ctx)
+        dfeature = torch.zeros((s.sdf.shape[0], 32), device=s.sdf.device) if dfeature is None else f32c(dfeature)
         dsdf = None if dsdf is None else f32c(dsdf)
         dalpha = None if dalpha is None else f32c(dalpha)
-        dx, dtable, dbeta, dws, dbs = _field_fused_backward(ctx, ctx.saved_tensors, dfeature, None, None, dsdf, dalpha)
-        return (dtable, dx, None, None, None, None, None, None, None, dbeta, *dws, *dbs, *ctx.dactor)
+        dx, grads = _field_fused_backward(ctx, s, dfeature, None, None, dsdf, dalpha)
+        return (grads[0], dx, None, None, None, None, None, None, None, *grads[1:])
 
 
 def field_fused(table: Optional[Tensor], x: Optional[Tensor], x3: Optional[Tensor], std: Optional[Tensor], sh: Tensor,
@@ -582,13 +605,11 @@ class _FieldRender(torch.autograd.Function):
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
     def forward(ctx, table, x3, std, sh, iv: "SampleIntervals", beta_min: float, spec, trans_eps: float, actors, beta, *params):
-        ctx.sink = grad_sink_of(table)
         train = any(ctx.needs_input_grad)
         ctx.needs_x_grad = False
-        sinks = [grad_sink_of(beta)] + [grad_sink_of(q) for q in params[:10]]
         S = iv.num_samples
-        feature, sdf, alpha = _field_fused_forward(ctx, table, None, x3, std, sh, S, beta_min, spec, beta, params, train, sinks,
-                                                   actors)
+        feature, sdf, alpha, saved = _field_fused_forward(ctx, table, None, x3, std, sh, S, beta_min, spec, beta, params, train,
+                                                          actors)
         N, dev = alpha.shape[0] // S, alpha.device
         weights = torch.empty((N, S), device=dev, dtype=torch.float32)
         features = torch.empty((N, 32), device=dev, dtype=torch.float32)
@@ -597,28 +618,27 @@ class _FieldRender(torch.autograd.Function):
         i = iv.struct()
         _lib.call("nrb_alpha_composite_fwd", ptr(alpha), ptr(feature), C.byref(i), N, 32, float(trans_eps), 1, ptr(weights),
                   ptr(features), ptr(depth), ptr(acc), None, stream_ptr())
-        if train:
-            ctx.render = (feature, weights, iv, float(trans_eps))
+        if train:  # (`weights` is an output: saved, not kept on ctx, so that output -> graph -> output is no cycle)
+            _save(ctx, **saved, feature=feature, render_weights=weights)
+            ctx.iv, ctx.trans_eps = iv, float(trans_eps)
         return weights, features, depth, acc
 
     @staticmethod
     @custom_bwd(device_type="cuda")
     def backward(ctx, dweights, dfeatures, ddepth, dacc):
-        feature, weights, iv, eps = ctx.render
-        alpha = ctx.saved_tensors[8]
-        N, S = weights.shape
-        dev = weights.device
+        s = _saved(ctx)
+        N, S = s.render_weights.shape
+        dev = s.render_weights.device
         dweights = None if dweights is None else f32c(dweights)
         dfeatures = torch.zeros((N, 32), device=dev) if dfeatures is None else f32c(dfeatures)
         ddepth = None if ddepth is None else f32c(ddepth)
         dacc = None if dacc is None else f32c(dacc)
         dalphas = torch.empty((N * S,), device=dev, dtype=torch.float32)
-        i = iv.struct()
-        _lib.call("nrb_alpha_composite_bwd", ptr(alpha), ptr(feature), C.byref(i), N, 32, eps, 1, ptr(dweights), ptr(dfeatures),
-                  ptr(ddepth), ptr(dacc), ptr(dalphas), None, stream_ptr())
-        _, dtable, dbeta, dws, dbs = _field_fused_backward(ctx, ctx.saved_tensors, None, dfeatures, weights.reshape(-1), None,
-                                                           dalphas)
-        return (dtable, None, None, None, None, None, None, None, None, dbeta, *dws, *dbs, *ctx.dactor)
+        i = ctx.iv.struct()
+        _lib.call("nrb_alpha_composite_bwd", ptr(s.alpha), ptr(s.feature), C.byref(i), N, 32, ctx.trans_eps, 1, ptr(dweights),
+                  ptr(dfeatures), ptr(ddepth), ptr(dacc), ptr(dalphas), None, stream_ptr())
+        _, grads = _field_fused_backward(ctx, s, None, dfeatures, s.render_weights.reshape(-1), None, dalphas)
+        return (grads[0], None, None, None, None, None, None, None, None, *grads[1:])
 
 
 def field_render(table: Tensor, x3: Tensor, std: Optional[Tensor], sh: Tensor, iv: SampleIntervals, spec: GridSpec,
@@ -952,8 +972,7 @@ class _ProposalRound(torch.autograd.Function):
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
     def forward(ctx, table, decoder_w, rays: RayData, iv: SampleIntervals, spec: GridSpec, scale: float, actors, *actor_tables):
-        ctx.sink = grad_sink_of(table)
-        ctx.dec_sink = grad_sink_of(decoder_w)
+        ctx.sinks = _GradSinks([table, decoder_w, *actor_tables])
         table = f32c(table)
         dec = f32c(decoder_w.reshape(-1))
         N, S = rays.num_rays, iv.num_samples
@@ -966,49 +985,38 @@ class _ProposalRound(torch.autograd.Function):
         g, r, i = spec.struct(table), rays.struct(), iv.struct()
         ag = asmp = None
         if actors is not None:
-            ctx.actor_sinks = [grad_sink_of(t) for t in actor_tables]
-            actors = ActorBatch(actors.grid_id, actors.pos, actors.std, actors.dirs, [f32c(t) for t in actor_tables], actors.spec)
+            actors = actors.with_tables([f32c(t) for t in actor_tables])
             ag, asmp = actors.grids_struct(), actors.samples_struct()
         _lib.call("nrb_proposal_fwd", C.byref(r), C.byref(g), ptr(dec), float(scale), C.byref(i), ptr(density),
                   ptr(weights), ptr(feats), ptr(pre), None if ag is None else C.byref(ag),
                   None if asmp is None else C.byref(asmp), stream_ptr())
-        extra = [] if actors is None else [actors.grid_id, actors.pos, actors.std, actors.dirs, *actors.tables]
-        ctx.save_for_backward(table, dec, feats, pre, *extra)
+        _save(ctx, table=table, dec=dec, feats=feats, pre=pre, actors=[] if actors is None else actors.to_save())
         ctx.rays, ctx.iv, ctx.spec, ctx.scale = rays, iv, spec, float(scale)
         ctx.actor_spec = None if actors is None else actors.spec
-        ctx.dec_shape = decoder_w.shape
         return density, weights
 
     @staticmethod
     @custom_bwd(device_type="cuda")
     def backward(ctx, ddensity, dweights):
-        table, dec, feats, pre, *extra = ctx.saved_tensors
-        dtable = ctx.sink if ctx.sink is not None else torch.zeros_like(table)
-        ddec = ctx.dec_sink.reshape(-1) if ctx.dec_sink is not None else torch.zeros_like(dec)
+        s, sinks = _saved(ctx), ctx.sinks
+        dtable, ddec = sinks.dest(0), sinks.dest(1)  # (ddec has the decoder's shape; the kernel reads it flat)
         ddensity = None if ddensity is None else f32c(ddensity)
         dweights = None if dweights is None else f32c(dweights)
-        g, r, i = ctx.spec.struct(table), ctx.rays.struct(), ctx.iv.struct()
+        g, r, i = ctx.spec.struct(s.table), ctx.rays.struct(), ctx.iv.struct()
         n_pts = ctx.rays.num_rays * ctx.iv.num_samples
-        ws, ws_bytes = _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(g), n_pts)), table.device)
+        ws, ws_bytes = _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(g), n_pts)), s.table.device)
         ag = asmp = dptrs = None
-        dactor: List[Optional[Tensor]] = []
+        dactor: List[Tensor] = []
         if ctx.actor_spec is not None:
-            actors = ActorBatch(extra[0], extra[1], extra[2], extra[3], list(extra[4:]), ctx.actor_spec)
+            actors = ActorBatch.from_saved(s.actors, ctx.actor_spec)
             ag, asmp = actors.grids_struct(), actors.samples_struct()
-            dactor = [sk if sk is not None else torch.zeros_like(t) for t, sk in zip(actors.tables, ctx.actor_sinks)]
+            dactor = [sinks.dest(i) for i in range(2, len(sinks.params))]
             dptrs = (C.c_void_p * len(dactor))(*[d.data_ptr() for d in dactor])
-        _lib.call("nrb_proposal_bwd", C.byref(r), C.byref(g), ptr(dec), ctx.scale, C.byref(i), ptr(feats), ptr(pre),
+        _lib.call("nrb_proposal_bwd", C.byref(r), C.byref(g), ptr(s.dec), ctx.scale, C.byref(i), ptr(s.feats), ptr(s.pre),
                   ptr(dweights), ptr(ddensity), ptr(dtable), ptr(ddec), ws, ws_bytes, None if ag is None else C.byref(ag),
                   None if asmp is None else C.byref(asmp), dptrs, stream_ptr())
-        if ctx.sink is not None:
-            _sink_written(table)
-        if ctx.actor_spec is not None:
-            for t, sk in zip(actors.tables, ctx.actor_sinks):
-                if sk is not None:
-                    _sink_written(t)
-            dactor = [None if sk is not None else d for d, sk in zip(dactor, ctx.actor_sinks)]
-        return ((None if ctx.sink is not None else dtable), (None if ctx.dec_sink is not None else ddec.reshape(ctx.dec_shape)),
-                None, None, None, None, None, *dactor)
+        grads = sinks.written([dtable, ddec, *dactor])
+        return (grads[0], grads[1], None, None, None, None, None, *grads[2:])
 
 
 def proposal_round(

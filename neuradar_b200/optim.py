@@ -13,51 +13,36 @@ from __future__ import annotations
 from typing import Dict, Iterable, List, Optional
 
 import torch
-import torch.distributed as dist
 from torch import Tensor
 
 from . import _lib
 from ._lib import AdamCfg, ptr, stream_ptr
-from .dist import OverlappedReduce, order_early_first, peer_memory_or_none
+from .dist import GradArena, padded_numel
 
 import ctypes as C
 
 
 class _FlatGroup:
-    """Parameters of one group re-homed into one flat buffer; .grad of each is a view of the flat gradient."""
+    """Parameters of one group re-homed into one flat buffer `p`, with Adam's moments `m` and `v` at the same offsets.
+    The gradients are a GradArena over the same parameters in the same order: `g` is its flat buffer."""
 
     def __init__(self, params: List[torch.nn.Parameter], direct_scatter: bool = False, early=None):
-        params, n_first = order_early_first(params, early if direct_scatter else None)
-        dev = params[0].device
-        offsets, total, n_early = [], 0, 0
-        for i, p in enumerate(params):
-            if p.dtype != torch.float32 or p.device != dev or not p.is_cuda:
-                raise ValueError("FusedAdam expects fp32 CUDA parameters on one device (there is no CPU path)")
-            offsets.append(total)
-            total += (p.numel() + 3) // 4 * 4  # 16-byte aligned views (vector atomics of the scatter kernels)
-            if i < n_first:
-                n_early = total
-        self.params, self.offsets, self.numel = params, offsets, total
-        self.p = torch.zeros((total,), device=dev, dtype=torch.float32)
-        self.peer = peer_memory_or_none(total, dev)  # data-parallel on one box: gradients in symmetric memory (dist.py)
-        self.g = self.peer.flat if self.peer is not None else torch.zeros_like(self.p)
+        if not all(p.is_cuda for p in params):
+            raise ValueError("FusedAdam expects fp32 CUDA parameters on one device (there is no CPU path)")
+        # p before g: their placement shows in the field backward's gradient flush (B200, config 2 with the optimizer:
+        # nrb_field_fused_bwd 0.84 ms with g allocated first, 0.82 ms this way)
+        self.numel = sum(padded_numel(p.numel()) for p in params)
+        self.p = torch.zeros((self.numel,), device=params[0].device, dtype=torch.float32)
+        self.arena = GradArena(params, direct_scatter=direct_scatter, early=early)
+        self.params, self.offsets, self.g = self.arena.params, self.arena.offsets, self.arena.flat
         self.m = torch.zeros_like(self.p)
         self.v = torch.ones_like(self.p)  # padding lanes keep v = 1 so that eps = 0 cannot make them 0 / 0
-        self.skipped = torch.zeros((1,), device=dev, dtype=torch.float32)  # steps GradScaler skipped (found_inf)
-        self.reducer = OverlappedReduce(self.g, n_early, self.peer)
-        for i, (p, off) in enumerate(zip(params, offsets)):
+        self.skipped = torch.zeros((1,), device=self.g.device, dtype=torch.float32)  # steps GradScaler skipped (found_inf)
+        for p, off in zip(self.params, self.offsets):
             self.v[off : off + p.numel()].zero_()
             view = self.p[off : off + p.numel()].view_as(p)
             view.copy_(p.data)
             p.data = view
-            gview = self.g[off : off + p.numel()].view_as(p)
-            if p.grad is not None:
-                gview.copy_(p.grad)
-            p.grad = gview
-            if direct_scatter:
-                p._nrb_grad_sink = gview  # the backward kernels add straight into the flat gradient
-                if i < n_first:
-                    p._nrb_grad_ready = self.reducer.start_early
 
 
 class FusedAdam(torch.optim.Optimizer):
@@ -76,6 +61,10 @@ class FusedAdam(torch.optim.Optimizer):
             ps = [p for p in group["params"] if p.requires_grad]
             self._flat.append(_FlatGroup(ps, direct_scatter, early))
             group["step"] = 0
+        if any(f.arena.peer is None for f in self._flat):  # all groups take one route, so one multiplier serves them all
+            for f in self._flat:
+                if f.arena.peer is not None:
+                    f.arena.reducer.use_nccl()
         # GradScaler.step sets (and deletes) self.grad_scale / self.found_inf around step(); they must not pre-exist
 
     # ---- the flat views (data parallelism reduces `flat_grads()` with one collective per group)
@@ -87,14 +76,14 @@ class FusedAdam(torch.optim.Optimizer):
 
     def zero_grad(self, set_to_none: bool = False) -> None:  # gradients stay views of the flat buffer
         for f in self._flat:
-            f.g.zero_()
+            f.arena.zero()
 
     def all_reduce_grads(self, group=None) -> float:
-        """Sum gradients over ranks; returns the multiplier (1 / world_size) for step(grad_mult=...)."""
-        mult = 1.0
-        for f in self._flat:  # gradients flagged `early` may already be in flight (dist.OverlappedReduce)
-            mult = f.reducer.finish(group)
-        return mult
+        """Sum gradients over the ranks of the default process group; returns the multiplier for step(grad_mult=...):
+        1 / world_size after NCCL, 1 after the peer-memory kernel (which averages in place)."""
+        mults = {f.arena.reduce(group) for f in self._flat}  # (the `early` gradients may already be in flight)
+        assert len(mults) == 1, f"parameter groups reduced by different routes: multipliers {mults}"
+        return mults.pop()
 
     def check_finite(self, found_inf: Optional[Tensor] = None) -> Tensor:
         """Device flag (1.0 if any gradient is inf / nan), like GradScaler's per-optimizer found_inf."""
@@ -117,16 +106,7 @@ class FusedAdam(torch.optim.Optimizer):
                     view = f.p[off : off + p.numel()].view_as(p)
                     view.copy_(p.data)
                     p.data = view
-                # someone replaced .grad (e.g. zero_grad(set_to_none=True))
-                if p.grad is None or p.grad.data_ptr() != f.g.data_ptr() + 4 * off:
-                    gview = f.g[off : off + p.numel()].view_as(p)
-                    if p.grad is not None:
-                        gview.copy_(p.grad)
-                    else:
-                        gview.zero_()
-                    p.grad = gview
-                    if getattr(p, "_nrb_grad_sink", None) is not None:
-                        p._nrb_grad_sink = gview
+            f.arena.relink()  # someone replaced .grad (e.g. zero_grad(set_to_none=True))
             group["step"] += 1
             cfg = AdamCfg(float(group["lr"]), float(group["betas"][0]), float(group["betas"][1]), float(group["eps"]),
                           float(group["weight_decay"]), int(self._decoupled), int(group["step"]), float(grad_mult),

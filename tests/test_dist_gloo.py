@@ -139,3 +139,54 @@ def test_early_overlapped_reduce_matches_single_collective(tmp_path):
     assert float(f0[74:76].abs().sum()) == 0.0                                # padding stays zero
     assert torch.allclose(f0[76:81], torch.full((5,), 15.0))
     assert torch.allclose(f0[84:93], torch.full((9,), 150.0))
+
+
+def _misuse_worker(rank: int, world: int, port: int, out_dir: str) -> None:
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    try:
+        from neuradar_b200._lib import NeuradarB200Error
+
+        table = torch.nn.Parameter(torch.zeros(8))
+        other = torch.nn.Parameter(torch.zeros(4))
+        arena = GradArena([other, table], direct_scatter=True, early=[table])
+        arena.zero()
+        # two backward passes per reduce (gradient accumulation, or two losses with retain_graph): the second write to
+        # the early region lands after its collective was launched and would never be exchanged
+        table._nrb_grad_sink.add_(float(rank + 1))
+        table._nrb_grad_ready()
+        table._nrb_grad_sink.add_(float(rank + 1))
+        with pytest.raises(NeuradarB200Error, match="gradient accumulation"):
+            table._nrb_grad_ready()
+        arena.all_reduce(average=True)  # joins the first collective; the reducer is idle again
+        assert arena.reducer._work is None
+        subgroup = dist.new_group([0, 1])  # the same ranks, but not the default group
+        with pytest.raises(ValueError):
+            arena.all_reduce(group=subgroup)
+    finally:
+        dist.destroy_process_group()
+
+
+def test_second_early_write_per_reduce_raises(tmp_path):
+    world = 2
+    mp.spawn(_misuse_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
+
+
+def test_single_process_early_writes_accumulate():
+    """Without data parallelism the early callback does nothing, so gradient accumulation keeps working."""
+    table = torch.nn.Parameter(torch.zeros(6))
+    arena = GradArena([table], direct_scatter=True, early=[table])
+    for k in (1.0, 2.0):
+        table._nrb_grad_sink.add_(k)
+        table._nrb_grad_ready()
+    arena.all_reduce()
+    assert torch.equal(table.grad, torch.full((6,), 3.0))
+
+
+def test_arena_keeps_an_existing_grad():
+    p = torch.nn.Parameter(torch.zeros(5))
+    p.grad = torch.arange(5.0)
+    arena = GradArena([p])
+    assert p.grad.data_ptr() == arena.flat.data_ptr()
+    assert torch.equal(p.grad, torch.arange(5.0))

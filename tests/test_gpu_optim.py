@@ -182,3 +182,66 @@ def test_direct_scatter_from_a_side_stream_is_ordered_before_the_default_stream(
         loss.backward()
         got = arena.flat[: want.numel()].clone()  # queued on the default stream immediately after backward()
         assert rel_err(got.view_as(want), want) <= 1e-5
+
+
+def test_decoder_only_sink_from_a_side_stream_is_ordered_before_the_default_stream():
+    """A proposal round on a side stream whose only gradient sink is its density decoder's (the "fields" optimiser
+    scatters directly, the "hashgrids" one does not): no gradient goes back to autograd, so only the sink bookkeeping
+    orders the decoder's gradient before work queued on the default stream right after `backward()`."""
+    from neuradar_b200 import functional as Fn
+    from neuradar_b200.dist import GradArena
+    from tests.parity_utils import build_hot_path, scaled_pixel_area, synthetic_rays
+
+    N, S = 16384, 64  # ~1 M samples: a backward long enough for a missing dependency to show
+    model = build_hot_path(log2_main=12, log2_prop=17, table_gain=(300.0, 2000.0), seed=4, device=DEV)
+    pf = model.proposal_fields[1]
+    table, dec = pf.hashgrid.static_grid.hash_table, pf.density_decoder.weight
+    table.requires_grad_(False)
+    rays = synthetic_rays(N, seed=6)
+    g = torch.Generator().manual_seed(3)
+    _, eb, _ = O.spaced_bins(rays["nears"], rays["fars"].clamp_max(20000.0), S, torch.rand((N, S + 1), generator=g))
+    rd = Fn.RayData(rays["origins"].to(DEV), rays["directions"].to(DEV), scaled_pixel_area(rays).to(DEV))
+    iv = Fn.SampleIntervals.from_bins(eb.contiguous().to(DEV))
+    gw = torch.randn((N, S), generator=g).to(DEV)
+
+    def loss():
+        _, w = Fn.proposal_round(table, dec, rd, iv, pf.hashgrid.static_grid.spec, 100.0)
+        return (w * gw).sum()
+
+    loss().backward()  # expected: ordinary autograd accumulation on the default stream
+    want = dec.grad.clone()
+    dec.grad = None
+    arena = GradArena([dec], direct_scatter=True)
+    side = torch.cuda.Stream()
+    for _ in range(3):
+        arena.zero()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            l = loss()
+        torch.cuda.current_stream().wait_stream(side)
+        l.backward()
+        got = arena.flat[: want.numel()].clone()  # queued on the default stream immediately after backward()
+        assert rel_err(got.view_as(want), want) <= 1e-4
+
+
+def test_field_render_keeps_no_reference_cycle():
+    """The outputs of `field_render` are saved for its backward, not kept on ctx: with the cyclic garbage collector off,
+    dropping the outputs after backward frees them (and the [M,32] feature buffer the node holds)."""
+    import gc
+    import weakref
+
+    from tests.parity_utils import build_hot_path, make_ray_bundle, synthetic_rays
+
+    model = build_hot_path(log2_main=12, log2_prop=12, table_gain=(300.0, 2000.0), seed=9, device=DEV)
+    rays = synthetic_rays(256, seed=10)
+    _, eb, _ = O.spaced_bins(rays["nears"], rays["fars"].clamp_max(20000.0), 48, torch.rand((256, 49)))
+    rs = make_ray_bundle(rays, DEV).get_ray_samples(bin_starts=eb[:, :-1, None].to(DEV), bin_ends=eb[:, 1:, None].to(DEV))
+    gc.disable()
+    try:
+        weights, features, depth, acc = model.field.render(rs)
+        alive = weakref.ref(weights)
+        (weights.sum() + features.sum() + depth.sum()).backward()
+        del weights, features, depth, acc
+        assert alive() is None
+    finally:
+        gc.enable()
