@@ -109,14 +109,14 @@ struct ActorGradDev {
   float* tables[NRB_MAX_ACTORS];
 };
 
-// Scatter of the 16 actor features' gradient (tile-image layout of field_fused.cu: chunk c of sample m at float4 index
-// (m / 128 * 8 + c) * 128 + m % 128) into the sample's actor table; optionally the gradient with respect to the sample's
-// position in the grid's unit cube.  One thread per (sample, level); ~10 % of the samples belong to actors.
+// Scatter of the 16 actor features' gradient (tile image of the fused field backward, tile_image_chunk) into the
+// sample's actor table; optionally the gradient with respect to the sample's position in the grid's unit cube.  One
+// thread per (sample, level); ~10 % of the samples belong to actors.
 template <bool kNeedDx>
 __global__ void __launch_bounds__(256) actor_scatter_kernel(const __grid_constant__ ActorGridsDev ag,
                                                             const __grid_constant__ ActorGradDev grads,
                                                             const __grid_constant__ ActorSamplesDev as,
-                                                            const float4* __restrict__ dyimg, float* __restrict__ dpos,
+                                                            const float* __restrict__ dyimg, float* __restrict__ dpos,
                                                             int64_t total) {
   const int64_t gid = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (gid >= total) return;
@@ -127,35 +127,27 @@ __global__ void __launch_bounds__(256) actor_scatter_kernel(const __grid_constan
   const float scal = ag.scalings[l];
   const float px = as.pos[3 * m], py = as.pos[3 * m + 1], pz = as.pos[3 * m + 2];
   const Cell c = locate_cell(px, py, pz, scal, (1u << ag.log2_size) - 1u);
-  const float4 g4 = __ldg(dyimg + ((m >> 7) * 8 + l) * 128 + (m & 127));  // features 4l .. 4l+3
+  float gr[4];
+  load_row<4>(tile_image_chunk(dyimg, m, l), 0, gr);  // features 4l .. 4l+3
   const float lw = level_weight(scal, as.std[m]);
-  const float gr[4] = {g4.x * lw, g4.y * lw, g4.z * lw, g4.w * lw};
+#pragma unroll
+  for (int j = 0; j < 4; ++j) gr[j] *= lw;
   float w[8];
   corner_weights(c, w);
   const size_t level_off = (static_cast<size_t>(l) << ag.log2_size) * 4;
   float* dt = grads.tables[grid] + level_off;
 #pragma unroll
-  for (int k = 0; k < 8; ++k) scatter_row<4>(dt, c.row[k], gr, w[k]);
+  for (int k = 0; k < 8; ++k) {
+    float v[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] = gr[j] * w[k];
+    scatter_row<4>(dt, c.row[k], v);
+  }
   if constexpr (kNeedDx) {
-    const float* tb = ag.tables[grid] + level_off;
-    float f[8][4];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) load_row<4>(tb, c.row[k], f[k]);
-    const float ax = c.ox, bx = 1.0f - c.ox, ay = c.oy, by = 1.0f - c.oy, az = c.oz, bz = 1.0f - c.oz;
-    float gx = 0.f, gy = 0.f, gz = 0.f;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float f03 = f[0][j] * ax + f[3][j] * bx, f12 = f[1][j] * ax + f[2][j] * bx;
-      const float f56 = f[5][j] * ax + f[6][j] * bx, f47 = f[4][j] * ax + f[7][j] * bx;
-      const float f0312 = f03 * ay + f12 * by, f4756 = f47 * ay + f56 * by;
-      gz += gr[j] * (f0312 - f4756);
-      gy += gr[j] * ((f03 - f12) * az + (f47 - f56) * bz);
-      gx += gr[j] * (((f[0][j] - f[3][j]) * ay + (f[1][j] - f[2][j]) * by) * az +
-                     ((f[4][j] - f[7][j]) * ay + (f[5][j] - f[6][j]) * by) * bz);
-    }
-    atomicAdd(dpos + 3 * m + 0, gx * scal);
-    atomicAdd(dpos + 3 * m + 1, gy * scal);
-    atomicAdd(dpos + 3 * m + 2, gz * scal);
+    const float3 d = position_grad<4>(ag.tables[grid] + level_off, c, gr);
+    atomicAdd(dpos + 3 * m + 0, d.x * scal);
+    atomicAdd(dpos + 3 * m + 1, d.y * scal);
+    atomicAdd(dpos + 3 * m + 2, d.z * scal);
   }
 }
 
@@ -198,11 +190,9 @@ extern "C" int nrb_actor_scatter(const nrb_actor_grids_t* grids, float* const* d
   if (dpos != nullptr) {
     cudaError_t e = cudaMemsetAsync(dpos, 0, sizeof(float) * 3 * M, s);
     NRB_REQUIRE(e == cudaSuccess, static_cast<int>(e), "nrb_actor_scatter: memset failed: %s", cudaGetErrorString(e));
-    actor_scatter_kernel<true><<<blocks_for(total, 256), 256, 0, s>>>(to_dev(grids), gd, as,
-                                                                      reinterpret_cast<const float4*>(dyimg), dpos, total);
+    actor_scatter_kernel<true><<<blocks_for(total, 256), 256, 0, s>>>(to_dev(grids), gd, as, dyimg, dpos, total);
   } else {
-    actor_scatter_kernel<false><<<blocks_for(total, 256), 256, 0, s>>>(to_dev(grids), gd, as,
-                                                                       reinterpret_cast<const float4*>(dyimg), dpos, total);
+    actor_scatter_kernel<false><<<blocks_for(total, 256), 256, 0, s>>>(to_dev(grids), gd, as, dyimg, dpos, total);
   }
   return finish_launch("nrb_actor_scatter");
 }

@@ -227,6 +227,34 @@ __device__ __forceinline__ void interpolate(const float* __restrict__ level_base
   }
 }
 
+// Gradient of one level's interpolated features with respect to the point's scaled position (x * scal), contracted
+// with the upstream values g: the derivative of `interpolate` above.  Multiply by the level's scaling for the point.
+template <int F>
+__device__ __forceinline__ float3 position_grad(const float* __restrict__ level_base, const Cell& c, const float (&g)[F]) {
+  float f[8][F];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) load_row<F>(level_base, c.row[k], f[k]);
+  const float ax = c.ox, bx = 1.0f - c.ox, ay = c.oy, by = 1.0f - c.oy, az = c.oz, bz = 1.0f - c.oz;
+  float gx = 0.f, gy = 0.f, gz = 0.f;
+#pragma unroll
+  for (int j = 0; j < F; ++j) {
+    const float f03 = f[0][j] * ax + f[3][j] * bx, f12 = f[1][j] * ax + f[2][j] * bx;
+    const float f56 = f[5][j] * ax + f[6][j] * bx, f47 = f[4][j] * ax + f[7][j] * bx;
+    const float f0312 = f03 * ay + f12 * by, f4756 = f47 * ay + f56 * by;
+    gz += g[j] * (f0312 - f4756);
+    gy += g[j] * ((f03 - f12) * az + (f47 - f56) * bz);
+    gx += g[j] * (((f[0][j] - f[3][j]) * ay + (f[1][j] - f[2][j]) * by) * az +
+                  ((f[4][j] - f[7][j]) * ay + (f[5][j] - f[6][j]) * by) * bz);
+  }
+  return make_float3(gx, gy, gz);
+}
+
+// The fused field backward's data-gradient tile image: [tile of 128 samples][8 chunks of 4 features][128 samples]
+// float4.  Returns features 4c .. 4c+3 of sample m; a warp of consecutive samples reads 16-byte-strided, i.e. coalesced.
+__device__ __forceinline__ const float* tile_image_chunk(const float* img, int64_t m, int c) {
+  return img + ((m >> 7) * 1024 + (m & 127)) * 4 + c * 512;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);

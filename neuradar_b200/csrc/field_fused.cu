@@ -929,59 +929,6 @@ __global__ void __maxnreg__(128) field_fused_bwd_kernel(const __grid_constant__ 
   if (uwarp == 0) tmem_free<512>(tmem_base);
 }
 
-// ---------------------------------------------------------------------------------------------------------------
-// Hash-grid gradient scatter reading the data gradient in the tile image the kernel above writes
-// ([tile][chunk of 4 features][128 samples] float4): a lane's level reads are 16-byte-strided across the warp, i.e.
-// coalesced, with no shared-memory staging.  Otherwise identical to hash_bwd_dedup_kernel (hash_grid.cu).
-// ---------------------------------------------------------------------------------------------------------------
-template <int F>
-__global__ void __launch_bounds__(256) hash_bwd_img_kernel(const __grid_constant__ GridDev g,
-                                                           const __grid_constant__ BwdPlan plan,
-                                                           const float* __restrict__ x, const float* __restrict__ std,
-                                                           const float* __restrict__ dyimg, float* __restrict__ dtable,
-                                                           const int32_t* __restrict__ actor_grid_id, int64_t M) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int L = g.num_levels;
-  const int64_t base = (static_cast<int64_t>(blockIdx.x) * 8 + warp) * 32;
-  if (base >= M) return;
-  const int64_t m = base + lane;
-  const int64_t mc = m < M ? m : (M - 1);
-  // samples claimed by an actor grid took none of their features from this table
-  const bool valid = m < M && (actor_grid_id == nullptr || __ldg(actor_grid_id + mc) < 0);
-  const float px = __ldg(x + 3 * mc), py = __ldg(x + 3 * mc + 1), pz = __ldg(x + 3 * mc + 2);
-  const float sd = std != nullptr ? __ldg(std + mc) : 0.0f;
-  const float* row = dyimg + ((m >> 7) * 1024 + (m & 127)) * 4;  // chunk c of this sample at row + c * 512 floats
-  const uint32_t mask = (1u << g.log2_size) - 1u;
-  const unsigned spread = static_cast<unsigned>(base >> 5);
-  for (int l = 0; l < L; ++l) {
-    const float scal = g.scalings[l];
-    const Cell c = locate_cell(px, py, pz, scal, mask);
-    float gr[F];
-    {
-      const int f0 = l * F;
-      const float* p = row + (f0 >> 2) * 512 + (f0 & 3);
-      if constexpr (F == 4) {
-        const float4 t4 = __ldg(reinterpret_cast<const float4*>(p));
-        gr[0] = t4.x, gr[1] = t4.y, gr[2] = t4.z, gr[3] = t4.w;
-      } else if constexpr (F == 2) {
-        const float2 t2 = __ldg(reinterpret_cast<const float2*>(p));
-        gr[0] = t2.x, gr[1] = t2.y;
-      } else {
-        gr[0] = __ldg(p);
-      }
-    }
-    const float lw = (std != nullptr ? level_weight(scal, sd) : 1.0f) * (valid ? 1.0f : 0.0f);
-    float w[8];
-    corner_weights(c, w);
-    float v[8][F];
-#pragma unroll
-    for (int k = 0; k < 8; ++k)
-#pragma unroll
-      for (int j = 0; j < F; ++j) v[k][j] = w[k] * (gr[j] * lw);
-    merge_runs_and_scatter<F>(plan, l, g.log2_size, px, py, pz, scal, c, v, valid, lane, dtable, spread);
-  }
-}
-
 }  // namespace nrb
 
 using namespace nrb;
@@ -1125,36 +1072,6 @@ extern "C" int nrb_field_fused_bwd(const nrb_field_mlp_t* p, const nrb_field_fus
   const unsigned nblk = static_cast<unsigned>(std::min<int64_t>((tiles + 1) / 2, sm_count()));
   field_fused_bwd_kernel<<<nblk, kBThreads, FusedBwdSmem::total, static_cast<cudaStream_t>(stream)>>>(fused_params(p), a, map);
   return finish_launch("nrb_field_fused_bwd");
-}
-
-extern "C" int nrb_hash_bwd_image(const nrb_grid_t* grid, const float* x, const float* std, const float* dyimg,
-                                  float* dtable, const int32_t* actor_grid_id, int64_t M, void* workspace,
-                                  int64_t workspace_bytes, nrb_stream_t stream) {
-  if (int rc = check_grid(grid)) return rc;
-  NRB_REQUIRE(x && dyimg && dtable && M >= 0, NRB_ERR_BAD_ARG, "nrb_hash_bwd_image: null pointer or negative M");
-  NRB_REQUIRE(aligned16(dyimg) && aligned16(dtable), NRB_ERR_ALIGNMENT, "nrb_hash_bwd_image: dyimg/dtable must be 16-byte aligned");
-  NRB_REQUIRE(grid->num_levels * grid->features_per_level == 32, NRB_ERR_UNSUPPORTED,
-              "nrb_hash_bwd_image: the tile image holds 32 features per sample");
-  if (M == 0) return NRB_OK;
-  auto s = static_cast<cudaStream_t>(stream);
-  BwdPlan plan;
-  int64_t vertices = 0;
-  if (int rc = prepare_bwd_plan(grid, M, workspace, workspace_bytes, s, &plan, &vertices)) return rc;
-  const GridDev g = to_dev(grid);
-  const unsigned nblk = blocks_for(M, 256);
-  switch (grid->features_per_level) {
-    case 2:
-      hash_bwd_img_kernel<2><<<nblk, 256, 0, s>>>(g, plan, x, std, dyimg, dtable, actor_grid_id, M);
-      launch_fold<2>(grid, plan, dtable, vertices, s);
-      break;
-    case 4:
-      hash_bwd_img_kernel<4><<<nblk, 256, 0, s>>>(g, plan, x, std, dyimg, dtable, actor_grid_id, M);
-      launch_fold<4>(grid, plan, dtable, vertices, s);
-      break;
-    default:
-      NRB_REQUIRE(false, NRB_ERR_UNSUPPORTED, "nrb_hash_bwd_image: features_per_level must be 2 or 4");
-  }
-  return finish_launch("nrb_hash_bwd_image");
 }
 
 #ifdef NRB_FUSED_TRACE

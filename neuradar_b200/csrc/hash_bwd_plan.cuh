@@ -3,7 +3,6 @@
 #pragma once
 
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -25,26 +24,13 @@ inline GridDev to_dev(const nrb_grid_t* g) {
   return d;
 }
 
-template <int F>
-__device__ __forceinline__ void scatter_row(float* __restrict__ base, uint32_t row, const float g[F], float w) {
-  float* p = base + static_cast<size_t>(row) * F;
-  if constexpr (F == 1) {
-    atomicAdd(p, g[0] * w);
-  } else if constexpr (F == 2) {
-    atomicAdd(reinterpret_cast<float2*>(p), make_float2(g[0] * w, g[1] * w));
-  } else {
-    atomicAdd(reinterpret_cast<float4*>(p), make_float4(g[0] * w, g[1] * w, g[2] * w, g[3] * w));
-  }
-}
-
 // Backward scatter.  Same-row float reductions serialise in L2: 25 M reductions take 0.16 ms when they spread over
 // the 2^19 rows of a res-1024 level and 7 ms when they pile onto the 4913 rows of a res-16 level (measured, B200).
 // Coarse levels are therefore accumulated into `copies[l]` replicas of the level's dense vertex lattice
 // ((res+1)^3 x F floats, a few MB in total, L2 resident); warps are dealt round-robin over the replicas, which
 // divides the per-address contention by the replica count, and a small fold kernel adds the replicas into the
-// hashed rows.  Levels that already fill the table but whose samples are still spatially coherent (res 84..256 at
-// T = 2^19) get a few replicas of the hashed level table itself.  Replica counts were swept on B200 (tools_bwd_sweep.py,
-// config 2): 8.5 ms without replicas, 3.9 ms with lattice replicas only, 2.7-2.8 ms with the defaults below.  Shared-memory privatisation was measured and rejected: fp32 shared atomics are CAS loops
+// hashed rows.  Levels that already fill the table scatter straight into it (DESIGN.md section 4 has the measurements
+// behind the plan).  Shared-memory privatisation was measured and rejected: fp32 shared atomics are CAS loops
 // (ATOMS.CAST.SPIN) on sm_100 and cost ~1 ms per level.
 struct BwdPlan {
   float* scratch;                   // replicated lattices, zeroed by the launcher
@@ -54,78 +40,10 @@ struct BwdPlan {
   int r1[NRB_MAX_LEVELS];           // res + 1
 };
 
-// Two rows that differ only in the x corner (floor / ceil).  The x prime of the hash is 1, so whenever floor(x) is
-// even the two rows are r and r ^ 1: an aligned pair of adjacent table rows.  For F <= 2 the pair is then updated with
-// ONE reduction of twice the width (F32x2 for F = 1, F32x4 for F = 2) - the L2 reduction rate is per operation, not
-// per byte, so this removes a quarter of the operations on average.  The same holds for the dense lattice replicas
-// (x neighbours are adjacent, aligned when the lower index is even).
+// The scatter works on per-corner VALUES: contributions already multiplied by their corner weights (and, in the
+// run-merging kernels, summed over a run of samples that share a cell).
 template <int F>
-__device__ __forceinline__ void scatter_x_pair(float* __restrict__ base, uint32_t row_f, uint32_t row_c,
-                                               const float (&g)[F], float w_f, float w_c) {
-  if constexpr (F <= 2) {
-    if (row_c == (row_f ^ 1u)) {
-      const bool f_low = (row_f & 1u) == 0;
-      const float wl = f_low ? w_f : w_c, wh = f_low ? w_c : w_f;
-      float* p = base + static_cast<size_t>(row_f & ~1u) * F;
-      if constexpr (F == 1) {
-        atomicAdd(reinterpret_cast<float2*>(p), make_float2(g[0] * wl, g[0] * wh));
-      } else {
-        atomicAdd(reinterpret_cast<float4*>(p), make_float4(g[0] * wl, g[1] * wl, g[0] * wh, g[1] * wh));
-      }
-      return;
-    }
-  }
-  scatter_row<F>(base, row_f, g, w_f);
-  if (row_c != row_f || w_c != 0.0f) scatter_row<F>(base, row_c, g, w_c);
-}
-
-// corner order (common.cuh): 0:(c,c,c) 1:(c,f,c) 2:(f,f,c) 3:(f,c,c) 4:(c,c,f) 5:(c,f,f) 6:(f,f,f) 7:(f,c,f);
-// x pairs (floor, ceil): (3,0) (2,1) (7,4) (6,5)
-template <int F>
-__device__ __forceinline__ void scatter_rows8(float* __restrict__ base, const uint32_t (&row)[8], const float (&g)[F],
-                                              const float (&w)[8]) {
-  scatter_x_pair<F>(base, row[3], row[0], g, w[3], w[0]);
-  scatter_x_pair<F>(base, row[2], row[1], g, w[2], w[1]);
-  scatter_x_pair<F>(base, row[7], row[4], g, w[7], w[4]);
-  scatter_x_pair<F>(base, row[6], row[5], g, w[6], w[5]);
-}
-
-// Scatter the 8 corner contributions of one (point, level): into a replica when the level is replicated (and the
-// point lies inside the lattice), otherwise straight into the table.  `spread` picks the replica (warp index).
-template <int F>
-__device__ __forceinline__ void scatter_corners(const BwdPlan& plan, int l, int log2_size, float scal, float px, float py,
-                                                float pz, const Cell& c, const float (&gr)[F], const float (&w)[8],
-                                                float* __restrict__ dtable, unsigned spread) {
-  const int copies = plan.copies[l];
-  if (copies > 1 && plan.r1[l] == 0) {  // replicas of the hashed level table
-    float* rep = plan.scratch + plan.offset[l] + static_cast<size_t>(spread % static_cast<unsigned>(copies)) * plan.stride[l];
-    scatter_rows8<F>(rep, c.row, gr, w);
-    return;
-  }
-  if (copies > 1) {  // replicas of the dense vertex lattice
-    const int R1 = plan.r1[l];
-    const float sx = mul(px, scal), sy = mul(py, scal), sz = mul(pz, scal);
-    const int xf = static_cast<int>(floorf(sx)), yf = static_cast<int>(floorf(sy)), zf = static_cast<int>(floorf(sz));
-    const int xc = static_cast<int>(ceilf(sx)), yc = static_cast<int>(ceilf(sy)), zc = static_cast<int>(ceilf(sz));
-    if (xf >= 0 && yf >= 0 && zf >= 0 && xc < R1 && yc < R1 && zc < R1) {
-      float* rep = plan.scratch + plan.offset[l] + static_cast<size_t>(spread % static_cast<unsigned>(copies)) * plan.stride[l];
-      const int cx[8] = {xc, xc, xf, xf, xc, xc, xf, xf};
-      const int cy[8] = {yc, yf, yf, yc, yc, yf, yf, yc};
-      const int cz[8] = {zc, zc, zc, zc, zf, zf, zf, zf};
-      uint32_t rows[8];
-#pragma unroll
-      for (int k = 0; k < 8; ++k) rows[k] = static_cast<uint32_t>((cz[k] * R1 + cy[k]) * R1 + cx[k]);
-      scatter_rows8<F>(rep, rows, gr, w);
-      return;
-    }
-  }
-  scatter_rows8<F>(dtable + (static_cast<size_t>(l) << log2_size) * F, c.row, gr, w);
-}
-
-// ---- the same scatter with per-corner VALUES (contributions already multiplied by their weights and summed over a run
-// of samples that share a cell, see hash_bwd_dedup_kernel)
-template <int F>
-__device__ __forceinline__ void scatter_row_v(float* __restrict__ base, uint32_t row, const float (&v)[F]) {
+__device__ __forceinline__ void scatter_row(float* __restrict__ base, uint32_t row, const float (&v)[F]) {
   float* p = base + static_cast<size_t>(row) * F;
   if constexpr (F == 1) {
     atomicAdd(p, v[0]);
@@ -136,14 +54,19 @@ __device__ __forceinline__ void scatter_row_v(float* __restrict__ base, uint32_t
   }
 }
 
+// Two rows that differ only in the x corner (floor / ceil).  The x prime of the hash is 1, so whenever floor(x) is
+// even the two rows are r and r ^ 1: an aligned pair of adjacent table rows.  For F <= 2 the pair is then updated with
+// ONE reduction of twice the width (F32x2 for F = 1, F32x4 for F = 2) - the L2 reduction rate is per operation, not
+// per byte, so this removes a quarter of the operations on average.  The same holds for the dense lattice replicas
+// (x neighbours are adjacent, aligned when the lower index is even).
 template <int F>
-__device__ __forceinline__ void scatter_x_pair_v(float* __restrict__ base, uint32_t row_f, uint32_t row_c,
-                                                 const float (&vf)[F], const float (&vc)[F]) {
+__device__ __forceinline__ void scatter_x_pair(float* __restrict__ base, uint32_t row_f, uint32_t row_c,
+                                               const float (&vf)[F], const float (&vc)[F]) {
   if (row_c == row_f) {  // integral x (ceil == floor; the ceil weight is 0) or a hash collision: one reduction
     float t[F];
 #pragma unroll
     for (int j = 0; j < F; ++j) t[j] = vf[j] + vc[j];
-    scatter_row_v<F>(base, row_f, t);
+    scatter_row<F>(base, row_f, t);
     return;
   }
   if constexpr (F <= 2) {
@@ -159,29 +82,28 @@ __device__ __forceinline__ void scatter_x_pair_v(float* __restrict__ base, uint3
       return;
     }
   }
-  scatter_row_v<F>(base, row_f, vf);
-  scatter_row_v<F>(base, row_c, vc);
+  scatter_row<F>(base, row_f, vf);
+  scatter_row<F>(base, row_c, vc);
 }
 
+// corner order (common.cuh): 0:(c,c,c) 1:(c,f,c) 2:(f,f,c) 3:(f,c,c) 4:(c,c,f) 5:(c,f,f) 6:(f,f,f) 7:(f,c,f);
+// x pairs (floor, ceil): (3,0) (2,1) (7,4) (6,5)
 template <int F>
-__device__ __forceinline__ void scatter_rows8_v(float* __restrict__ base, const uint32_t (&row)[8], const float (&v)[8][F]) {
-  scatter_x_pair_v<F>(base, row[3], row[0], v[3], v[0]);
-  scatter_x_pair_v<F>(base, row[2], row[1], v[2], v[1]);
-  scatter_x_pair_v<F>(base, row[7], row[4], v[7], v[4]);
-  scatter_x_pair_v<F>(base, row[6], row[5], v[6], v[5]);
+__device__ __forceinline__ void scatter_rows8(float* __restrict__ base, const uint32_t (&row)[8], const float (&v)[8][F]) {
+  scatter_x_pair<F>(base, row[3], row[0], v[3], v[0]);
+  scatter_x_pair<F>(base, row[2], row[1], v[2], v[1]);
+  scatter_x_pair<F>(base, row[7], row[4], v[7], v[4]);
+  scatter_x_pair<F>(base, row[6], row[5], v[6], v[5]);
 }
 
-// (xf, yf, zf) / (xc, yc, zc): integer floor / ceil coordinates of the cell (for the dense lattice replicas)
+// Scatter the 8 corner values of one (point, level): into a replica when the level is replicated and the point lies
+// inside the lattice, otherwise straight into the table.  (xf, yf, zf) / (xc, yc, zc): integer floor / ceil
+// coordinates of the cell; `spread` picks the replica (warp index).
 template <int F>
-__device__ __forceinline__ void scatter_corners_v(const BwdPlan& plan, int l, int log2_size, int xf, int yf, int zf, int xc,
-                                                  int yc, int zc, const uint32_t (&hashed_rows)[8], const float (&v)[8][F],
-                                                  float* __restrict__ dtable, unsigned spread) {
+__device__ __forceinline__ void scatter_corners(const BwdPlan& plan, int l, int log2_size, int xf, int yf, int zf, int xc,
+                                                int yc, int zc, const uint32_t (&hashed_rows)[8], const float (&v)[8][F],
+                                                float* __restrict__ dtable, unsigned spread) {
   const int copies = plan.copies[l];
-  if (copies > 1 && plan.r1[l] == 0) {
-    float* rep = plan.scratch + plan.offset[l] + static_cast<size_t>(spread % static_cast<unsigned>(copies)) * plan.stride[l];
-    scatter_rows8_v<F>(rep, hashed_rows, v);
-    return;
-  }
   if (copies > 1) {
     const int R1 = plan.r1[l];
     if (xf >= 0 && yf >= 0 && zf >= 0 && xc < R1 && yc < R1 && zc < R1) {
@@ -192,11 +114,11 @@ __device__ __forceinline__ void scatter_corners_v(const BwdPlan& plan, int l, in
       uint32_t rows[8];
 #pragma unroll
       for (int k = 0; k < 8; ++k) rows[k] = static_cast<uint32_t>((cz[k] * R1 + cy[k]) * R1 + cx[k]);
-      scatter_rows8_v<F>(rep, rows, v);
+      scatter_rows8<F>(rep, rows, v);
       return;
     }
   }
-  scatter_rows8_v<F>(dtable + (static_cast<size_t>(l) << log2_size) * F, hashed_rows, v);
+  scatter_rows8<F>(dtable + (static_cast<size_t>(l) << log2_size) * F, hashed_rows, v);
 }
 
 // Run merging (called by all 32 lanes of a converged warp whose lanes hold CONSECUTIVE samples of a ray): lanes whose
@@ -236,70 +158,16 @@ __device__ __forceinline__ void merge_runs_and_scatter(const BwdPlan& plan, int 
     }
     issue = valid && head;
   }
-  if (issue) scatter_corners_v<F>(plan, l, log2_size, xf, yf, zf, xc, yc, zc, c.row, v, dtable, spread);
+  if (issue) scatter_corners<F>(plan, l, log2_size, xf, yf, zf, xc, yc, zc, c.row, v, dtable, spread);
 }
 
-// Adds the replicas of every replicated level into the table: one thread per lattice vertex.
-template <int F>
-__global__ void __launch_bounds__(256) hash_bwd_fold_kernel(const __grid_constant__ GridDev g,
-                                                            const __grid_constant__ BwdPlan plan,
-                                                            float* __restrict__ dtable, int64_t total_vertices) {
-  int64_t v = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (v >= total_vertices) return;
-  int l = 0;
-  for (; l < g.num_levels; ++l) {
-    if (plan.copies[l] <= 1) continue;
-    const int64_t nvl = plan.r1[l] > 0 ? static_cast<int64_t>(plan.r1[l]) * plan.r1[l] * plan.r1[l]
-                                       : (int64_t{1} << g.log2_size);
-    if (v < nvl) break;
-    v -= nvl;
-  }
-  if (l >= g.num_levels) return;
-  const int R1 = plan.r1[l];
-  const int64_t nv = R1 > 0 ? static_cast<int64_t>(R1) * R1 * R1 : (int64_t{1} << g.log2_size);
-  const float* rep = plan.scratch + plan.offset[l] + v * F;
-  float sum[F];
-#pragma unroll
-  for (int j = 0; j < F; ++j) sum[j] = 0.0f;
-  for (int cpy = 0; cpy < plan.copies[l]; ++cpy) {
-    float t[F];
-    load_row<F>(rep + static_cast<size_t>(cpy) * plan.stride[l], 0, t);
-#pragma unroll
-    for (int j = 0; j < F; ++j) sum[j] += t[j];
-  }
-  bool any = false;
-#pragma unroll
-  for (int j = 0; j < F; ++j) any |= (sum[j] != 0.0f);
-  if (!any) return;
-  uint32_t row;
-  if (R1 > 0) {
-    const int ix = static_cast<int>(v % R1), iy = static_cast<int>((v / R1) % R1), iz = static_cast<int>(v / (R1 * R1));
-    row = (static_cast<uint32_t>(ix) ^ (static_cast<uint32_t>(iy) * kPrimeY) ^ (static_cast<uint32_t>(iz) * kPrimeZ)) &
-          ((1u << g.log2_size) - 1u);
-  } else {
-    row = static_cast<uint32_t>(v);
-  }
-  scatter_row<F>(dtable + (static_cast<size_t>(l) << g.log2_size) * F, row, sum, 1.0f);
-}
-
-inline double env_or(const char* name, double dflt) {
-  const char* v = std::getenv(name);
-  return v != nullptr ? std::atof(v) : dflt;
-}
-
+// Dense-lattice replicas for the coarse levels: copies ~ table rows / lattice vertices, at most 32 MiB per level
+// (DESIGN.md section 4).  Levels whose lattice is not much smaller than the table get none.
 inline int64_t plan_hash_bwd(const nrb_grid_t* grid, int64_t M, BwdPlan* plan) {
-  // Tunables, swept on B200 at config 2 (tools/sweep_bwd_env*.sh; DESIGN.md section 4).  Dense-lattice replicas for the
-  // coarse levels: copies ~ scale * table_rows / vertices, at most cap_mb per level.  Replicas of the HASHED level
-  // tables (hashed > 1) paid off before run merging (3.2 -> 2.4 ms); with it they only cost L2 capacity, so they are off
-  // by default and remain available for sample orders that do not merge (NRB_BWD_HASHED_COPIES / _LEVELS).
-  static const double scale = env_or("NRB_BWD_SCALE", 1.0), cap_mb = env_or("NRB_BWD_CAP_MB", 32.0);
-  static const int hashed = static_cast<int>(env_or("NRB_BWD_HASHED_COPIES", 1.0));
-  static const int hashed_levels = static_cast<int>(env_or("NRB_BWD_HASHED_LEVELS", 4.0));
+  constexpr double kMaxBytesPerLevel = 32.0 * 1024 * 1024;
   const int F = grid->features_per_level;
-  const int64_t T = int64_t{1} << grid->log2_hashmap_size;
-  const double table_rows = static_cast<double>(T);
+  const double table_rows = static_cast<double>(int64_t{1} << grid->log2_hashmap_size);
   int64_t floats = 0;
-  int hashed_used = 0;
   for (int l = 0; l < NRB_MAX_LEVELS; ++l) {
     plan->copies[l] = 0;
     plan->offset[l] = 0;
@@ -308,28 +176,15 @@ inline int64_t plan_hash_bwd(const nrb_grid_t* grid, int64_t M, BwdPlan* plan) {
     if (l >= grid->num_levels || M < (int64_t{1} << 16)) continue;
     const int64_t r1 = static_cast<int64_t>(grid->scalings[l]) + 1;
     const double verts = static_cast<double>(r1) * r1 * r1;
-    int copies;
-    int64_t per_copy;
-    if (verts * 1.5 > table_rows || r1 > 1024) {  // the level already spreads over (most of) the table
-      if (hashed <= 1 || hashed_used >= hashed_levels) continue;
-      ++hashed_used;
-      copies = hashed;
-      per_copy = T * F;
-      plan->r1[l] = 0;  // replicas of the hashed level table
-    } else {
-      copies = static_cast<int>(scale * table_rows / verts + 0.5);
-      copies = std::min(copies, 1024);
-      per_copy = (r1 * r1 * r1 * F + 3) & ~int64_t{3};
-      plan->r1[l] = static_cast<int>(r1);
-    }
-    while (copies > 1 && static_cast<double>(copies) * per_copy * 4 > cap_mb * 1024 * 1024) --copies;
-    if (copies <= 1) {
-      plan->r1[l] = 0;
-      continue;
-    }
+    if (verts * 1.5 > table_rows || r1 > 1024) continue;  // the level already spreads over (most of) the table
+    const int64_t per_copy = (r1 * r1 * r1 * F + 3) & ~int64_t{3};
+    int copies = std::min(static_cast<int>(table_rows / verts + 0.5), 1024);
+    while (copies > 1 && static_cast<double>(copies) * per_copy * 4 > kMaxBytesPerLevel) --copies;
+    if (copies <= 1) continue;
     plan->copies[l] = copies;
     plan->stride[l] = per_copy;
     plan->offset[l] = floats;
+    plan->r1[l] = static_cast<int>(r1);
     floats += static_cast<int64_t>(copies) * per_copy;
     floats = (floats + 3) & ~int64_t{3};
   }
@@ -346,9 +201,7 @@ inline int prepare_bwd_plan(const nrb_grid_t* grid, int64_t M, void* workspace, 
     cudaError_t e = cudaMemsetAsync(workspace, 0, static_cast<size_t>(need), s);
     NRB_REQUIRE(e == cudaSuccess, static_cast<int>(e), "backward workspace memset failed: %s", cudaGetErrorString(e));
     for (int l = 0; l < grid->num_levels; ++l)
-      if (plan->copies[l] > 1)
-        *vertices += plan->r1[l] > 0 ? static_cast<int64_t>(plan->r1[l]) * plan->r1[l] * plan->r1[l]
-                                     : (int64_t{1} << grid->log2_hashmap_size);
+      if (plan->copies[l] > 1) *vertices += static_cast<int64_t>(plan->r1[l]) * plan->r1[l] * plan->r1[l];
   } else {  // no (or too small a) workspace: every level scatters straight into the table
     plan->scratch = nullptr;
     for (int l = 0; l < NRB_MAX_LEVELS; ++l) plan->copies[l] = 0;
@@ -356,11 +209,7 @@ inline int prepare_bwd_plan(const nrb_grid_t* grid, int64_t M, void* workspace, 
   return NRB_OK;
 }
 
-template <int F>
-inline void launch_fold(const nrb_grid_t* grid, const BwdPlan& plan, float* dtable, int64_t vertices, cudaStream_t s) {
-  if (vertices <= 0) return;
-  count_launch();
-  hash_bwd_fold_kernel<F><<<blocks_for(vertices, 256), 256, 0, s>>>(to_dev(grid), plan, dtable, vertices);
-}
+// Adds the replicas of every replicated level into the table (hash_grid.cu); nothing to do when `vertices` is 0.
+void launch_fold(const nrb_grid_t* grid, const BwdPlan& plan, float* dtable, int64_t vertices, cudaStream_t s);
 
 }  // namespace nrb

@@ -46,7 +46,7 @@ __global__ void __launch_bounds__(256) hash_fwd_kernel(const __grid_constant__ G
 }
 
 // Sample-major forward: one warp = 32 consecutive samples (lane = sample), looping over the levels.  Consecutive
-// samples of a ray mostly fall into the same cell (see hash_bwd_dedup_kernel), so the 32 gathers of one corner hit a
+// samples of a ray mostly fall into the same cell (see hash_bwd_merge_kernel), so the 32 gathers of one corner hit a
 // handful of distinct rows and coalesce in L1/TEX, which is the unit that bounds the level-major kernel above (ncu:
 // 95 % busy, one line per lane).  The 32 output rows are assembled in a swizzled shared-memory tile and written with
 // coalesced 16-byte stores.
@@ -122,50 +122,30 @@ __global__ void __launch_bounds__(256) hash_bwd_kernel(const __grid_constant__ G
   const float scal = g.scalings[l];
   const float px = __ldg(x + 3 * m), py = __ldg(x + 3 * m + 1), pz = __ldg(x + 3 * m + 2);
   const Cell c = locate_cell(px, py, pz, scal, (1u << g.log2_size) - 1u);
-  using V = typename Feat<F>::type;
-  const V gv = __ldg(reinterpret_cast<const V*>(dy) + gid);
   float gr[F];
-  if constexpr (F == 1) {
-    gr[0] = gv;
-  } else if constexpr (F == 2) {
-    gr[0] = gv.x;
-    gr[1] = gv.y;
-  } else {
-    gr[0] = gv.x;
-    gr[1] = gv.y;
-    gr[2] = gv.z;
-    gr[3] = gv.w;
-  }
+  load_row<F>(dy + gid * F, 0, gr);
   if (std != nullptr) {
     const float lw = level_weight(scal, __ldg(std + m));
 #pragma unroll
     for (int j = 0; j < F; ++j) gr[j] *= lw;
   }
-  const size_t level_off = (static_cast<size_t>(l) << g.log2_size) * F;
-  if constexpr (kNeedDx) {
-    // d out / d offset needs the corner features themselves.
-    float f[8][F];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) load_row<F>(g.table + level_off, c.row[k], f[k]);
-    const float ax = c.ox, bx = 1.0f - c.ox, ay = c.oy, by = 1.0f - c.oy, az = c.oz, bz = 1.0f - c.oz;
-    float gx = 0.f, gy = 0.f, gz = 0.f;
-#pragma unroll
-    for (int j = 0; j < F; ++j) {
-      const float f03 = f[0][j] * ax + f[3][j] * bx, f12 = f[1][j] * ax + f[2][j] * bx;
-      const float f56 = f[5][j] * ax + f[6][j] * bx, f47 = f[4][j] * ax + f[7][j] * bx;
-      const float f0312 = f03 * ay + f12 * by, f4756 = f47 * ay + f56 * by;
-      gz += gr[j] * (f0312 - f4756);
-      gy += gr[j] * ((f03 - f12) * az + (f47 - f56) * bz);
-      gx += gr[j] * (((f[0][j] - f[3][j]) * ay + (f[1][j] - f[2][j]) * by) * az +
-                     ((f[4][j] - f[7][j]) * ay + (f[5][j] - f[6][j]) * by) * bz);
-    }
-    atomicAdd(dx + 3 * m + 0, gx * scal);
-    atomicAdd(dx + 3 * m + 1, gy * scal);
-    atomicAdd(dx + 3 * m + 2, gz * scal);
+  if constexpr (kNeedDx) {  // d out / d offset needs the corner features themselves
+    const float3 d = position_grad<F>(g.table + (static_cast<size_t>(l) << g.log2_size) * F, c, gr);
+    atomicAdd(dx + 3 * m + 0, d.x * scal);
+    atomicAdd(dx + 3 * m + 1, d.y * scal);
+    atomicAdd(dx + 3 * m + 2, d.z * scal);
   }
   float w[8];
   corner_weights(c, w);
-  scatter_corners<F>(plan, l, g.log2_size, scal, px, py, pz, c, gr, w, dtable, static_cast<unsigned>(gid >> 5));
+  float v[8][F];
+#pragma unroll
+  for (int k = 0; k < 8; ++k)
+#pragma unroll
+    for (int j = 0; j < F; ++j) v[k][j] = w[k] * gr[j];
+  const float sx = mul(px, scal), sy = mul(py, scal), sz = mul(pz, scal);
+  const int xf = static_cast<int>(floorf(sx)), yf = static_cast<int>(floorf(sy)), zf = static_cast<int>(floorf(sz));
+  const int xc = static_cast<int>(ceilf(sx)), yc = static_cast<int>(ceilf(sy)), zc = static_cast<int>(ceilf(sz));
+  scatter_corners<F>(plan, l, g.log2_size, xf, yf, zf, xc, yc, zc, c.row, v, dtable, static_cast<unsigned>(gid >> 5));
 }
 
 // Backward scatter with run merging.  One warp = 32 consecutive samples (lane = sample), looping over the levels.
@@ -174,54 +154,62 @@ __global__ void __launch_bounds__(256) hash_bwd_kernel(const __grid_constant__ G
 // The scatter kernels are bound by the number of reductions they issue (RED issue rate, DESIGN.md section 4), so each
 // run of adjacent lanes with identical (floor, ceil) cell coordinates first adds up its 8 x F corner contributions with
 // a segmented shuffle reduction, and only the head lane of the run issues reductions (merge_runs_and_scatter,
-// hash_bwd_plan.cuh).  dy rows are staged through shared memory (coalesced loads, XOR-swizzled 16-byte chunks) because
-// a lane reading its own row touches 32 lines per load.
-constexpr int kDedupWarps = 8;
+// hash_bwd_plan.cuh).
+//   kImage = false: dy is row-major [M, L*F] (nrb_hash_bwd).  Its rows are staged through shared memory (coalesced
+//                   loads, XOR-swizzled 16-byte chunks) because a lane reading its own row touches 32 lines per load.
+//   kImage = true:  dy is the fused field backward's tile image (nrb_hash_bwd_image, tile_image_chunk), which a lane
+//                   reads coalesced without staging.  actor_grid_id (may be null) marks the samples claimed by an actor
+//                   grid: they took none of their features from this table.
+constexpr int kMergeWarps = 8;
 
-template <int F>
-__global__ void __launch_bounds__(kDedupWarps * 32) hash_bwd_dedup_kernel(const __grid_constant__ GridDev g,
+template <int F, bool kImage>
+__global__ void __launch_bounds__(kMergeWarps * 32) hash_bwd_merge_kernel(const __grid_constant__ GridDev g,
                                                                           const __grid_constant__ BwdPlan plan,
                                                                           const float* __restrict__ x,
                                                                           const float* __restrict__ std,
                                                                           const float* __restrict__ dy,
+                                                                          const int32_t* __restrict__ actor_grid_id,
                                                                           float* __restrict__ dtable, int64_t M) {
-  extern __shared__ __align__(16) char dedup_smem[];
+  extern __shared__ __align__(16) char dy_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int L = g.num_levels, RW = L * F;  // floats per dy row (4, 8, ..., 64: checked by the launcher)
   const int CPR = RW / 4;                  // 16-byte chunks per row
-  char* tile = dedup_smem + warp * (32 * RW * 4);
-  const int64_t base = (static_cast<int64_t>(blockIdx.x) * kDedupWarps + warp) * 32;
+  char* tile = dy_smem + warp * (32 * RW * 4);
+  const int64_t base = (static_cast<int64_t>(blockIdx.x) * kMergeWarps + warp) * 32;
   if (base >= M) return;
   const int64_t m = base + lane;
-  const bool valid = m < M;
-  const int64_t mc = valid ? m : (M - 1);
-  // coalesced copy of the 32 dy rows into the swizzled tile
-  for (int e = lane; e < 32 * CPR; e += 32) {
-    const int r = e / CPR, cc = e - r * CPR;
-    const int64_t rr = min(base + r, M - 1);
-    const float4 t = __ldg(reinterpret_cast<const float4*>(dy + rr * RW) + cc);
-    *reinterpret_cast<float4*>(tile + r * (RW * 4) + ((cc ^ (r % CPR)) << 4)) = t;
+  const int64_t mc = m < M ? m : (M - 1);
+  const bool valid = m < M && (!kImage || actor_grid_id == nullptr || __ldg(actor_grid_id + mc) < 0);
+  if constexpr (!kImage) {  // coalesced copy of the 32 dy rows into the swizzled tile
+    for (int e = lane; e < 32 * CPR; e += 32) {
+      const int r = e / CPR, cc = e - r * CPR;
+      const int64_t rr = min(base + r, M - 1);
+      const float4 t = __ldg(reinterpret_cast<const float4*>(dy + rr * RW) + cc);
+      *reinterpret_cast<float4*>(tile + r * (RW * 4) + ((cc ^ (r % CPR)) << 4)) = t;
+    }
   }
   const float px = __ldg(x + 3 * mc), py = __ldg(x + 3 * mc + 1), pz = __ldg(x + 3 * mc + 2);
   const float sd = std != nullptr ? __ldg(std + mc) : 0.0f;
-  __syncwarp();
+  if constexpr (!kImage) __syncwarp();
   const uint32_t mask = (1u << g.log2_size) - 1u;
   const unsigned spread = static_cast<unsigned>(base >> 5);
   for (int l = 0; l < L; ++l) {
     const float scal = g.scalings[l];
     const Cell c = locate_cell(px, py, pz, scal, mask);
+    const int f0 = l * F;  // first float of this level in the row
     float gr[F];
-    {
-      const int f0 = l * F;  // first float of this level in the row
-      const char* rowp = tile + lane * (RW * 4);
+    if constexpr (kImage) {
+      load_row<F>(tile_image_chunk(dy, m, f0 >> 2) + (f0 & 3), 0, gr);
+    } else {
+      const char* p = tile + lane * (RW * 4) + (((f0 >> 2) ^ (lane % CPR)) << 4) + (f0 & 3) * 4;
       if constexpr (F == 4) {
-        const float4 t = *reinterpret_cast<const float4*>(rowp + (((f0 >> 2) ^ (lane % CPR)) << 4));
+        const float4 t = *reinterpret_cast<const float4*>(p);
         gr[0] = t.x, gr[1] = t.y, gr[2] = t.z, gr[3] = t.w;
       } else if constexpr (F == 2) {
-        const float2 t = *reinterpret_cast<const float2*>(rowp + (((f0 >> 2) ^ (lane % CPR)) << 4) + (f0 & 3) * 4);
+        const float2 t = *reinterpret_cast<const float2*>(p);
         gr[0] = t.x, gr[1] = t.y;
       } else {
-        gr[0] = *reinterpret_cast<const float*>(rowp + (((f0 >> 2) ^ (lane % CPR)) << 4) + (f0 & 3) * 4);
+        gr[0] = *reinterpret_cast<const float*>(p);
       }
     }
     const float lw = (std != nullptr ? level_weight(scal, sd) : 1.0f) * (valid ? 1.0f : 0.0f);
@@ -233,6 +221,53 @@ __global__ void __launch_bounds__(kDedupWarps * 32) hash_bwd_dedup_kernel(const 
 #pragma unroll
       for (int j = 0; j < F; ++j) v[k][j] = w[k] * (gr[j] * lw);
     merge_runs_and_scatter<F>(plan, l, g.log2_size, px, py, pz, scal, c, v, valid, lane, dtable, spread);
+  }
+}
+
+// Adds the replicas of every replicated level into the table: one thread per lattice vertex.
+template <int F>
+__global__ void __launch_bounds__(256) hash_bwd_fold_kernel(const __grid_constant__ GridDev g,
+                                                            const __grid_constant__ BwdPlan plan,
+                                                            float* __restrict__ dtable, int64_t total_vertices) {
+  int64_t v = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (v >= total_vertices) return;
+  int l = 0;
+  for (; l < g.num_levels; ++l) {
+    if (plan.copies[l] <= 1) continue;
+    const int64_t nvl = static_cast<int64_t>(plan.r1[l]) * plan.r1[l] * plan.r1[l];
+    if (v < nvl) break;
+    v -= nvl;
+  }
+  if (l >= g.num_levels) return;
+  const float* rep = plan.scratch + plan.offset[l] + v * F;
+  float sum[F];
+#pragma unroll
+  for (int j = 0; j < F; ++j) sum[j] = 0.0f;
+  for (int cpy = 0; cpy < plan.copies[l]; ++cpy) {
+    float t[F];
+    load_row<F>(rep + static_cast<size_t>(cpy) * plan.stride[l], 0, t);
+#pragma unroll
+    for (int j = 0; j < F; ++j) sum[j] += t[j];
+  }
+  bool any = false;
+#pragma unroll
+  for (int j = 0; j < F; ++j) any |= (sum[j] != 0.0f);
+  if (!any) return;
+  const int R1 = plan.r1[l];
+  const int ix = static_cast<int>(v % R1), iy = static_cast<int>((v / R1) % R1), iz = static_cast<int>(v / (R1 * R1));
+  const uint32_t row = (static_cast<uint32_t>(ix) ^ (static_cast<uint32_t>(iy) * kPrimeY) ^
+                        (static_cast<uint32_t>(iz) * kPrimeZ)) & ((1u << g.log2_size) - 1u);
+  scatter_row<F>(dtable + (static_cast<size_t>(l) << g.log2_size) * F, row, sum);
+}
+
+void launch_fold(const nrb_grid_t* grid, const BwdPlan& plan, float* dtable, int64_t vertices, cudaStream_t s) {
+  if (vertices <= 0) return;
+  count_launch();
+  const unsigned blocks = blocks_for(vertices, 256);
+  switch (grid->features_per_level) {
+    case 1: hash_bwd_fold_kernel<1><<<blocks, 256, 0, s>>>(to_dev(grid), plan, dtable, vertices); break;
+    case 2: hash_bwd_fold_kernel<2><<<blocks, 256, 0, s>>>(to_dev(grid), plan, dtable, vertices); break;
+    default: hash_bwd_fold_kernel<4><<<blocks, 256, 0, s>>>(to_dev(grid), plan, dtable, vertices); break;
   }
 }
 
@@ -327,19 +362,17 @@ static int launch_hash_bwd(const nrb_grid_t* grid, const GridDev& g, const float
   const unsigned blocks = blocks_for(total, 256);
   const int row_floats = grid->num_levels * F;
   if (dx == nullptr && row_floats >= 4 && row_floats <= 64 && (row_floats & (row_floats - 1)) == 0 && M >= 32) {
-    const size_t smem = static_cast<size_t>(kDedupWarps) * 32 * row_floats * 4;
-    cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(hash_bwd_dedup_kernel<F>), 64 * 1024);
+    const size_t smem = static_cast<size_t>(kMergeWarps) * 32 * row_floats * 4;
+    cudaError_t e = ensure_dynamic_smem(reinterpret_cast<const void*>(hash_bwd_merge_kernel<F, false>), 64 * 1024);
     NRB_REQUIRE(e == cudaSuccess, static_cast<int>(e), "nrb_hash_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    hash_bwd_dedup_kernel<F><<<blocks_for(M, kDedupWarps * 32), kDedupWarps * 32, smem, s>>>(g, plan, x, std, dy, dtable, M);
-    launch_fold<F>(grid, plan, dtable, vertices, s);
-    return finish_launch("nrb_hash_bwd");
-  }
-  if (dx != nullptr) {
+    hash_bwd_merge_kernel<F, false><<<blocks_for(M, kMergeWarps * 32), kMergeWarps * 32, smem, s>>>(g, plan, x, std, dy,
+                                                                                                    nullptr, dtable, M);
+  } else if (dx != nullptr) {
     hash_bwd_kernel<F, true><<<blocks, 256, 0, s>>>(g, plan, x, std, dy, dtable, dx, total);
   } else {
     hash_bwd_kernel<F, false><<<blocks, 256, 0, s>>>(g, plan, x, std, dy, dtable, dx, total);
   }
-  launch_fold<F>(grid, plan, dtable, vertices, s);
+  launch_fold(grid, plan, dtable, vertices, s);
   return finish_launch("nrb_hash_bwd");
 }
 
@@ -360,6 +393,35 @@ extern "C" int nrb_hash_bwd(const nrb_grid_t* grid, const float* x, const float*
     case 2: return launch_hash_bwd<2>(grid, g, x, std, dy, dtable, dx, M, workspace, workspace_bytes, s);
     default: return launch_hash_bwd<4>(grid, g, x, std, dy, dtable, dx, M, workspace, workspace_bytes, s);
   }
+}
+
+extern "C" int nrb_hash_bwd_image(const nrb_grid_t* grid, const float* x, const float* std, const float* dyimg,
+                                  float* dtable, const int32_t* actor_grid_id, int64_t M, void* workspace,
+                                  int64_t workspace_bytes, nrb_stream_t stream) {
+  if (int rc = check_grid(grid)) return rc;
+  NRB_REQUIRE(x && dyimg && dtable && M >= 0, NRB_ERR_BAD_ARG, "nrb_hash_bwd_image: null pointer or negative M");
+  NRB_REQUIRE(aligned16(dyimg) && aligned16(dtable), NRB_ERR_ALIGNMENT, "nrb_hash_bwd_image: dyimg/dtable must be 16-byte aligned");
+  NRB_REQUIRE(grid->num_levels * grid->features_per_level == 32, NRB_ERR_UNSUPPORTED,
+              "nrb_hash_bwd_image: the tile image holds 32 features per sample");
+  if (M == 0) return NRB_OK;
+  auto s = static_cast<cudaStream_t>(stream);
+  BwdPlan plan;
+  int64_t vertices = 0;
+  if (int rc = prepare_bwd_plan(grid, M, workspace, workspace_bytes, s, &plan, &vertices)) return rc;
+  const GridDev g = to_dev(grid);
+  const unsigned nblk = blocks_for(M, kMergeWarps * 32);
+  switch (grid->features_per_level) {
+    case 2:
+      hash_bwd_merge_kernel<2, true><<<nblk, kMergeWarps * 32, 0, s>>>(g, plan, x, std, dyimg, actor_grid_id, dtable, M);
+      break;
+    case 4:
+      hash_bwd_merge_kernel<4, true><<<nblk, kMergeWarps * 32, 0, s>>>(g, plan, x, std, dyimg, actor_grid_id, dtable, M);
+      break;
+    default:
+      NRB_REQUIRE(false, NRB_ERR_UNSUPPORTED, "nrb_hash_bwd_image: features_per_level must be 2 or 4");
+  }
+  launch_fold(grid, plan, dtable, vertices, s);
+  return finish_launch("nrb_hash_bwd_image");
 }
 
 extern "C" int nrb_frustum_gaussians(const nrb_rays_t* rays, const nrb_intervals_t* iv, float scale, float* x,

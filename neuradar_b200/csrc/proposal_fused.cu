@@ -207,7 +207,12 @@ __global__ void __launch_bounds__(kPropWarps * 32) proposal_bwd_kernel(
             corner_weights(cell, w8);
             float* dt = g.adtables[agid] + (static_cast<size_t>(l) << g.ag.log2_size) * F;
 #pragma unroll
-            for (int k = 0; k < 8; ++k) scatter_row<F>(dt, cell.row[k], gr, w8[k]);
+            for (int k = 0; k < 8; ++k) {
+              float v[F];
+#pragma unroll
+              for (int j = 0; j < F; ++j) v[j] = gr[j] * w8[k];
+              scatter_row<F>(dt, cell.row[k], v);
+            }
           }
         }
         const bool act_static = act && agid < 0;
@@ -350,10 +355,6 @@ extern "C" int nrb_proposal_bwd(const nrb_rays_t* rays, const nrb_grid_t* grid, 
   }
 #undef NRB_LAUNCH
 #undef NRB_LAUNCH_C
-  switch (grid->features_per_level) {
-    case 1: launch_fold<1>(grid, plan, dtable, vertices, s); break;
-    case 2: launch_fold<2>(grid, plan, dtable, vertices, s); break;
-    default: launch_fold<4>(grid, plan, dtable, vertices, s); break;
-  }
+  launch_fold(grid, plan, dtable, vertices, s);
   return finish_launch("nrb_proposal_bwd");
 }

@@ -151,6 +151,11 @@ def _workspace(nbytes: int, device):
     return buf.data_ptr(), nbytes
 
 
+def _scatter_workspace(grid_struct: Grid, M: int, device):
+    """Workspace of a hash-table gradient scatter over M samples (the lattice replicas of its coarse levels)."""
+    return _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(grid_struct), M)), device)
+
+
 _SIDE_STREAMS = {}
 
 
@@ -291,7 +296,7 @@ class _HashEncode(torch.autograd.Function):
         dtable = ctx.sinks.dest(0)
         dx = torch.empty_like(x) if need_dx else None
         g = spec.struct(table)
-        ws, ws_bytes = _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(g), x.shape[0])), x.device)
+        ws, ws_bytes = _scatter_workspace(g, x.shape[0], x.device)
         _lib.call("nrb_hash_bwd", C.byref(g), ptr(x), ptr(std), ptr(dy), ptr(dtable), ptr(dx), x.shape[0], ws, ws_bytes,
                   stream_ptr(), tag="nrb_hash_bwd:" + spec.tag)
         return dx, *ctx.sinks.written([dtable]), None, None, None
@@ -503,7 +508,7 @@ def _field_fused_backward(ctx, s: SimpleNamespace, dfeature, dfeat_ray, weights,
         spec = ctx.spec
         dtable = sinks.dest(0)
         g = spec.struct(s.table)
-        ws, ws_bytes = _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(g), M)), dev)
+        ws, ws_bytes = _scatter_workspace(g, M, dev)
         _lib.call("nrb_hash_bwd_image", C.byref(g), ptr(s.x3), ptr(s.std), ptr(dximg), ptr(dtable),
                   None if actors is None else ptr(actors.grid_id), M, ws, ws_bytes, stream_ptr(), tag="nrb_hash_bwd:" + spec.tag)
     elif ctx.needs_x_grad:
@@ -1003,8 +1008,7 @@ class _ProposalRound(torch.autograd.Function):
         ddensity = None if ddensity is None else f32c(ddensity)
         dweights = None if dweights is None else f32c(dweights)
         g, r, i = ctx.spec.struct(s.table), ctx.rays.struct(), ctx.iv.struct()
-        n_pts = ctx.rays.num_rays * ctx.iv.num_samples
-        ws, ws_bytes = _workspace(int(_lib_().nrb_hash_bwd_workspace_bytes(C.byref(g), n_pts)), s.table.device)
+        ws, ws_bytes = _scatter_workspace(g, ctx.rays.num_rays * ctx.iv.num_samples, s.table.device)
         ag = asmp = dptrs = None
         dactor: List[Tensor] = []
         if ctx.actor_spec is not None:

@@ -58,16 +58,24 @@ def test_hash_indices_bit_exact(nb, golden):
     assert torch.equal(Fn.hash_indices(xo.to(DEV), spec).cpu(), want)
 
 
-@pytest.mark.parametrize("L,F,M", [(16, 2, 1000), (16, 2, 33), (16, 2, 31), (8, 4, 4097), (4, 4, 640), (6, 1, 500)])
-def test_hash_clustered_samples_run_merging(nb, L, F, M):
+@pytest.mark.parametrize(
+    "L,F,M,log2T,need_dx",
+    [pytest.param(L, F, M, 12, False, id=f"{L}-{F}-{M}")
+     for L, F, M in [(16, 2, 1000), (16, 2, 33), (16, 2, 31), (8, 4, 4097), (4, 4, 640), (6, 1, 500)]]
+    # T = 2^19 and M >= 2^16: the coarse levels scatter into dense-lattice replicas that a fold kernel adds up
+    + [(16, 2, 70000, 19, False), (8, 4, 66000, 19, False), (6, 1, 65600, 19, False), (12, 2, 65600, 19, True)],
+)
+def test_hash_clustered_samples_run_merging(nb, L, F, M, log2T, need_dx):
     """The sample-major forward and the run-merging backward on what they are built for: ray-ordered samples that
     pile into the same cells (identical points, integral coordinates, runs crossing warp boundaries), ragged M, and
-    the shapes that take the level-major fallback (M < 32, L*F not a power of two).  The table gradient must equal
-    the oracle's index_add whatever the grouping."""
+    the shapes that take the level-major fallback (M < 32, L*F not a power of two, x.grad requested).  The table
+    gradient must equal the oracle's index_add whatever the grouping, with and without lattice replicas."""
+    import ctypes as C
+
+    from neuradar_b200 import _lib
     from neuradar_b200 import functional as Fn
 
     g = torch.Generator().manual_seed(M + L)
-    log2T = 12
     anchors = torch.rand((max(M // 40, 1), 3), generator=g)
     x = anchors.repeat_interleave(40, dim=0)[:M].clone()
     if x.shape[0] < M:
@@ -81,13 +89,19 @@ def test_hash_clustered_samples_run_merging(nb, L, F, M):
     table = (torch.rand(((1 << log2T) * L, F), generator=g) * 2 - 1)
     dy = torch.randn((M, L * F), generator=g)
     t_ref = table.clone().requires_grad_(True)
-    y_ref = O.hash_encode(x, t_ref, scal, log2T)
+    x_ref = x.clone().requires_grad_(need_dx)
+    y_ref = O.hash_encode(x_ref, t_ref, scal, log2T)
     (y_ref * dy).sum().backward()
     t_dev = table.to(DEV).requires_grad_(True)
-    y = Fn.hash_encode(x.to(DEV), t_dev, spec)
+    x_dev = x.to(DEV).requires_grad_(need_dx)
+    if log2T == 19:
+        assert _lib.load().nrb_hash_bwd_workspace_bytes(C.byref(spec.struct(t_dev)), M) > 0
+    y = Fn.hash_encode(x_dev, t_dev, spec)
     assert rel_err(y, y_ref) <= 1e-6
     (y * dy.to(DEV)).sum().backward()
     assert rel_err(t_dev.grad, t_ref.grad) <= 1e-5  # fp32 sums in a different order
+    if need_dx:
+        assert rel_err(x_dev.grad, x_ref.grad) <= 1e-5
 
 
 @pytest.mark.parametrize("F", [1, 2, 4])
