@@ -54,14 +54,20 @@ __device__ __forceinline__ void scatter_row(float* __restrict__ base, uint32_t r
   }
 }
 
-// Two rows that differ only in the x corner (floor / ceil).  The x prime of the hash is 1, so whenever floor(x) is
-// even the two rows are r and r ^ 1: an aligned pair of adjacent table rows.  For F <= 2 the pair is then updated with
-// ONE reduction of twice the width (F32x2 for F = 1, F32x4 for F = 2) - the L2 reduction rate is per operation, not
-// per byte, so this removes a quarter of the operations on average.  The same holds for the dense lattice replicas
-// (x neighbours are adjacent, aligned when the lower index is even).
+// Two rows that differ only in the x corner (floor / ceil).  The x prime of the hash is 1, so the rows are
+// floor(x) ^ H and (floor(x) + 1) ^ H with the same H: they differ only in the low bits that the increment carries
+// into.  The L2 reduction rate is per operation, not per byte, so the pair is updated with ONE reduction whenever both
+// rows lie in one aligned 16-byte group:
+//   F = 1: rows r and r' with r >> 2 == r' >> 2 (floor(x) mod 4 != 3: 3 pairs in 4), one F32x4 whose other two slots
+//          add +0;
+//   F = 2: rows r and r ^ 1 (floor(x) even: 1 pair in 2), one F32x4.
+// That is 5 instead of 8 reductions per (point, level) on average for F = 1, 6 for F = 2.  The same holds for the dense
+// lattice replicas (x neighbours are adjacent; replicas are 16-byte aligned and padded to whole groups).  `quad`: the
+// level holds at least 4 rows, so a 16-byte group of F = 1 rows lies inside it and is aligned (only a 2-row table is
+// smaller).
 template <int F>
 __device__ __forceinline__ void scatter_x_pair(float* __restrict__ base, uint32_t row_f, uint32_t row_c,
-                                               const float (&vf)[F], const float (&vc)[F]) {
+                                               const float (&vf)[F], const float (&vc)[F], bool quad) {
   if (row_c == row_f) {  // integral x (ceil == floor; the ceil weight is 0) or a hash collision: one reduction
     float t[F];
 #pragma unroll
@@ -69,16 +75,19 @@ __device__ __forceinline__ void scatter_x_pair(float* __restrict__ base, uint32_
     scatter_row<F>(base, row_f, t);
     return;
   }
-  if constexpr (F <= 2) {
+  if constexpr (F == 1) {
+    if (quad && (row_f ^ row_c) < 4u) {
+      const uint32_t sf = row_f & 3u, sc = row_c & 3u;
+      const float4 t = make_float4(sf == 0 ? vf[0] : (sc == 0 ? vc[0] : 0.0f), sf == 1 ? vf[0] : (sc == 1 ? vc[0] : 0.0f),
+                                   sf == 2 ? vf[0] : (sc == 2 ? vc[0] : 0.0f), sf == 3 ? vf[0] : (sc == 3 ? vc[0] : 0.0f));
+      atomicAdd(reinterpret_cast<float4*>(base) + (row_f >> 2), t);
+      return;
+    }
+  } else if constexpr (F == 2) {
     if (row_c == (row_f ^ 1u)) {
       const bool f_low = (row_f & 1u) == 0;
-      float* p = base + static_cast<size_t>(row_f & ~1u) * F;
-      if constexpr (F == 1) {
-        atomicAdd(reinterpret_cast<float2*>(p), f_low ? make_float2(vf[0], vc[0]) : make_float2(vc[0], vf[0]));
-      } else {
-        atomicAdd(reinterpret_cast<float4*>(p), f_low ? make_float4(vf[0], vf[1], vc[0], vc[1])
-                                                      : make_float4(vc[0], vc[1], vf[0], vf[1]));
-      }
+      atomicAdd(reinterpret_cast<float4*>(base) + (row_f >> 1), f_low ? make_float4(vf[0], vf[1], vc[0], vc[1])
+                                                                     : make_float4(vc[0], vc[1], vf[0], vf[1]));
       return;
     }
   }
@@ -89,11 +98,12 @@ __device__ __forceinline__ void scatter_x_pair(float* __restrict__ base, uint32_
 // corner order (common.cuh): 0:(c,c,c) 1:(c,f,c) 2:(f,f,c) 3:(f,c,c) 4:(c,c,f) 5:(c,f,f) 6:(f,f,f) 7:(f,c,f);
 // x pairs (floor, ceil): (3,0) (2,1) (7,4) (6,5)
 template <int F>
-__device__ __forceinline__ void scatter_rows8(float* __restrict__ base, const uint32_t (&row)[8], const float (&v)[8][F]) {
-  scatter_x_pair<F>(base, row[3], row[0], v[3], v[0]);
-  scatter_x_pair<F>(base, row[2], row[1], v[2], v[1]);
-  scatter_x_pair<F>(base, row[7], row[4], v[7], v[4]);
-  scatter_x_pair<F>(base, row[6], row[5], v[6], v[5]);
+__device__ __forceinline__ void scatter_rows8(float* __restrict__ base, const uint32_t (&row)[8], const float (&v)[8][F],
+                                              bool quad) {
+  scatter_x_pair<F>(base, row[3], row[0], v[3], v[0], quad);
+  scatter_x_pair<F>(base, row[2], row[1], v[2], v[1], quad);
+  scatter_x_pair<F>(base, row[7], row[4], v[7], v[4], quad);
+  scatter_x_pair<F>(base, row[6], row[5], v[6], v[5], quad);
 }
 
 // Scatter the 8 corner values of one (point, level): into a replica when the level is replicated and the point lies
@@ -114,11 +124,11 @@ __device__ __forceinline__ void scatter_corners(const BwdPlan& plan, int l, int 
       uint32_t rows[8];
 #pragma unroll
       for (int k = 0; k < 8; ++k) rows[k] = static_cast<uint32_t>((cz[k] * R1 + cy[k]) * R1 + cx[k]);
-      scatter_rows8<F>(rep, rows, v);
+      scatter_rows8<F>(rep, rows, v, true);
       return;
     }
   }
-  scatter_rows8<F>(dtable + (static_cast<size_t>(l) << log2_size) * F, hashed_rows, v);
+  scatter_rows8<F>(dtable + (static_cast<size_t>(l) << log2_size) * F, hashed_rows, v, log2_size >= 2);
 }
 
 // Run merging (called by all 32 lanes of a converged warp whose lanes hold CONSECUTIVE samples of a ray): lanes whose

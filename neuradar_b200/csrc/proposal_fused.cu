@@ -109,34 +109,40 @@ __global__ void __launch_bounds__(kPropWarps * 32) proposal_fwd_kernel(
   }
 }
 
-// kChunks = ceil(S / 32) rounded up to 2 / 4 / 8: the per-chunk state of the two scans lives in registers, and a kernel
-// instantiated for 8 chunks carries 40 of them for nothing at S <= 64 (90 registers and 5 blocks per SM instead of 8).
+// Two phases.  (1) Warp per ray: the forward weight scan is recomputed from the saved pre-activations and the reverse
+// scan turns d weights into d density; kChunks = ceil(S / 32) rounded up to 2 / 4 / 8, because the per-chunk state of
+// the two scans lives in registers and a kernel instantiated for 8 chunks carries 40 of them for nothing at S <= 64.
+// Each sample's d pre (after trunc_exp) goes to shared memory.  (2) The block's rays_per_block * S samples, ray-major,
+// are cut into consecutive chunks of 32 and every warp scatters a contiguous range of them: a chunk may cross a ray
+// boundary, so S = 48 runs no idle lanes (one warp per ray would run a second chunk of 16).  Run merging stays exact
+// across the boundary: runs are formed on cell coordinates only, and two samples in one cell update the same rows
+// whichever ray they belong to.
 template <int F, int kChunks>
 __global__ void __launch_bounds__(kPropWarps * 32) proposal_bwd_kernel(
     const __grid_constant__ PropGrid g, const __grid_constant__ BwdPlan plan, const float* __restrict__ origins, const float* __restrict__ directions,
-    const float* __restrict__ pixel_area, float scale, nrb_intervals_t iv, int64_t N,
+    const float* __restrict__ pixel_area, float scale, nrb_intervals_t iv, int64_t N, int rays_per_block,
     const float* __restrict__ saved_feats, const float* __restrict__ saved_pre, const float* __restrict__ dweights,
     const float* __restrict__ ddensity, float* __restrict__ dtable, float* __restrict__ ddecoder) {
+  extern __shared__ float s_gpre[];  // [rays_per_block * S]
   __shared__ float s_ddec[NRB_MAX_LEVELS * 4];
   __shared__ float s_dec[NRB_MAX_LEVELS * 4];
   const int lane = threadIdx.x & 31;
+  const int warp = threadIdx.x >> 5;
   const int S = iv.num_samples;
   const int LF = g.num_levels * F;
   if (threadIdx.x < NRB_MAX_LEVELS * 4) {
     s_ddec[threadIdx.x] = 0.0f;
     s_dec[threadIdx.x] = threadIdx.x < LF ? g.decoder[threadIdx.x] : 0.0f;
   }
-  __syncthreads();
-  const int64_t n = static_cast<int64_t>(blockIdx.x) * kPropWarps + (threadIdx.x >> 5);
-  if (n < N) {
-    const float ox = origins[3 * n], oy = origins[3 * n + 1], oz = origins[3 * n + 2];
-    const float dx = directions[3 * n], dy = directions[3 * n + 1], dz = directions[3 * n + 2];
-    const float pa = pixel_area[n];
+  const int64_t n0 = static_cast<int64_t>(blockIdx.x) * rays_per_block;
+  const int rays = static_cast<int>(min(static_cast<int64_t>(rays_per_block), N - n0));
+#pragma unroll 1
+  for (int r = warp; r < rays; r += kPropWarps) {
+    const int64_t n = n0 + r;
     const float* st = iv.starts + n * iv.row_stride;
     const float* en = iv.ends + n * iv.row_stride;
-    const uint32_t mask = (1u << g.log2_size) - 1u;
     // forward recompute of the weight scan from the saved pre-activations
-    float delta[kChunks], dd[kChunks], trans[kChunks], pre[kChunks], gdens[kChunks];
+    float delta[kChunks], dd[kChunks], trans[kChunks], pre[kChunks];
     float carry = 0.0f;
 #pragma unroll
     for (int c = 0; c < kChunks; ++c) {
@@ -153,7 +159,7 @@ __global__ void __launch_bounds__(kPropWarps * 32) proposal_bwd_kernel(
         carry += __shfl_sync(kFull, incl, 31);
       }
     }
-    // d weights -> d density (reverse exclusive scan), see density_weights_bwd_kernel
+    // d weights -> d density (reverse exclusive scan), see density_weights_bwd_kernel, -> d pre (trunc_exp)
     float suffix = 0.0f;
 #pragma unroll
     for (int c = kChunks - 1; c >= 0; --c) {
@@ -172,75 +178,88 @@ __global__ void __launch_bounds__(kPropWarps * 32) proposal_bwd_kernel(
           if (lane + o < 32) incl += v;
         }
         float excl = __shfl_down_sync(kFull, incl, 1);
-      if (lane == 31) excl = 0.0f;
-      const float later = suffix + excl;
-        gdens[c] = ok ? (gwt * trans[c] * e - later) * delta[c] : 0.0f;
-        if (ok && ddensity != nullptr) gdens[c] += ddensity[n * S + i];
+        if (lane == 31) excl = 0.0f;
+        const float later = suffix + excl;
+        if (ok) {
+          float gdens = (gwt * trans[c] * e - later) * delta[c];
+          if (ddensity != nullptr) gdens += ddensity[n * S + i];
+          s_gpre[r * S + i] = gdens * expf(fminf(fmaxf(pre[c], -15.0f), 15.0f));
+        }
         suffix += __shfl_sync(kFull, incl, 0);
       }
     }
-    // d density -> d pre (trunc_exp) -> decoder and table gradients
-    const unsigned spread = static_cast<unsigned>(blockIdx.x * kPropWarps + (threadIdx.x >> 5));
-#pragma unroll
-    for (int c = 0; c < kChunks; ++c) {
-      if (c * 32 < S) {  // warp-uniform: all lanes take part in the run merging below
-        const int i = c * 32 + lane;
-        const bool act = i < S;
-        const int ic = act ? i : (S - 1);
-        const float gpre = act ? gdens[c] * expf(fminf(fmaxf(pre[c], -15.0f), 15.0f)) : 0.0f;
-        const Gaussian q = sample_gaussian(ox, oy, oz, dx, dy, dz, pa, st[ic], en[ic], scale);
-        const float* sf = saved_feats + (n * S + ic) * LF;
-        const int agid = g.agid != nullptr ? g.agid[n * S + ic] : -1;
-        if (act && agid >= 0) {  // the sample's gradient goes to its actor's table (plain reductions: ~10 % of the samples)
-          const float ax = g.apos[3 * (n * S + ic)], ay = g.apos[3 * (n * S + ic) + 1], az = g.apos[3 * (n * S + ic) + 2];
-          const float asd = g.astd[n * S + ic];
-          const uint32_t amask = (1u << g.ag.log2_size) - 1u;
-#pragma unroll
-          for (int l = 0; l < kActorLevels; ++l) {
-            const float scal = g.ag.scalings[l];
-            const Cell cell = locate_cell(ax, ay, az, scal, amask);
-            const float lw = level_weight(scal, asd);
-            float gr[F];
-#pragma unroll
-            for (int j = 0; j < F; ++j) gr[j] = gpre * s_dec[l * F + j] * lw;
-            float w8[8];
-            corner_weights(cell, w8);
-            float* dt = g.adtables[agid] + (static_cast<size_t>(l) << g.ag.log2_size) * F;
-#pragma unroll
-            for (int k = 0; k < 8; ++k) {
-              float v[F];
-#pragma unroll
-              for (int j = 0; j < F; ++j) v[j] = gr[j] * w8[k];
-              scatter_row<F>(dt, cell.row[k], v);
-            }
-          }
-        }
-        const bool act_static = act && agid < 0;
-        // A real loop over the levels: unrolled 16 x (with the chunks: up to 128 copies of the merge-and-scatter body)
-        // the kernel was 150 K instructions, far beyond the instruction cache.
+  }
+  __syncthreads();
+  // d pre -> decoder and table gradients, over the block's samples in chunks of 32
+  const int total = rays * S;
+  const int chunks = (total + 31) >> 5;
+  const int per_warp = (chunks + kPropWarps - 1) / kPropWarps;
+  const int c_end = min(chunks, (warp + 1) * per_warp);
+  const unsigned spread = static_cast<unsigned>(blockIdx.x * kPropWarps + warp);
+  const uint32_t mask = (1u << g.log2_size) - 1u;
 #pragma unroll 1
-        for (int l = 0; l < g.num_levels; ++l) {
-          const float scal = g.scalings[l];
-          const Cell cell = locate_cell(q.x, q.y, q.z, scal, mask);
-          const float lw = level_weight(scal, q.std);
-          float gr[F];
+  for (int c = warp * per_warp; c < c_end; ++c) {  // warp-uniform: all lanes take part in the run merging below
+    const int k = c * 32 + lane;
+    const bool act = k < total;
+    const int kc = act ? k : total - 1;
+    const int r = kc / S;
+    const int i = kc - r * S;
+    const int64_t n = n0 + r;
+    const int64_t m = n0 * S + kc;  // == n * S + i
+    const float gpre = act ? s_gpre[kc] : 0.0f;
+    const Gaussian q = sample_gaussian(origins[3 * n], origins[3 * n + 1], origins[3 * n + 2], directions[3 * n],
+                                       directions[3 * n + 1], directions[3 * n + 2], pixel_area[n],
+                                       iv.starts[n * iv.row_stride + i], iv.ends[n * iv.row_stride + i], scale);
+    const float* sf = saved_feats + m * LF;
+    const int agid = g.agid != nullptr ? g.agid[m] : -1;
+    if (act && agid >= 0) {  // the sample's gradient goes to its actor's table (plain reductions: ~10 % of the samples)
+      const float ax = g.apos[3 * m], ay = g.apos[3 * m + 1], az = g.apos[3 * m + 2];
+      const float asd = g.astd[m];
+      const uint32_t amask = (1u << g.ag.log2_size) - 1u;
 #pragma unroll
-          for (int j = 0; j < F; ++j) {
-            const float dd_lj = warp_sum(gpre * sf[l * F + j]);  // decoder gradient of this chunk's 32 samples
-            if (lane == 0) atomicAdd(&s_ddec[l * F + j], dd_lj);
-            gr[j] = gpre * s_dec[l * F + j] * lw;
-          }
-          float w8[8];
-          corner_weights(cell, w8);
-          // runs of adjacent samples of the ray that share a cell are summed before scattering (hash_bwd_plan.cuh)
-          float v[8][F];
+      for (int l = 0; l < kActorLevels; ++l) {
+        const float scal = g.ag.scalings[l];
+        const Cell cell = locate_cell(ax, ay, az, scal, amask);
+        const float lw = level_weight(scal, asd);
+        float gr[F];
 #pragma unroll
-          for (int k = 0; k < 8; ++k)
+        for (int j = 0; j < F; ++j) gr[j] = gpre * s_dec[l * F + j] * lw;
+        float w8[8];
+        corner_weights(cell, w8);
+        float* dt = g.adtables[agid] + (static_cast<size_t>(l) << g.ag.log2_size) * F;
 #pragma unroll
-            for (int j = 0; j < F; ++j) v[k][j] = w8[k] * gr[j];
-          merge_runs_and_scatter<F>(plan, l, g.log2_size, q.x, q.y, q.z, scal, cell, v, act_static, lane, dtable, spread);
+        for (int k8 = 0; k8 < 8; ++k8) {
+          float v[F];
+#pragma unroll
+          for (int j = 0; j < F; ++j) v[j] = gr[j] * w8[k8];
+          scatter_row<F>(dt, cell.row[k8], v);
         }
       }
+    }
+    const bool act_static = act && agid < 0;
+    // A real loop over the levels: unrolled 16 x (with the chunks: up to 128 copies of the merge-and-scatter body)
+    // the kernel was 150 K instructions, far beyond the instruction cache.
+#pragma unroll 1
+    for (int l = 0; l < g.num_levels; ++l) {
+      const float scal = g.scalings[l];
+      const Cell cell = locate_cell(q.x, q.y, q.z, scal, mask);
+      const float lw = level_weight(scal, q.std);
+      float gr[F];
+#pragma unroll
+      for (int j = 0; j < F; ++j) {
+        const float dd_lj = warp_sum(gpre * sf[l * F + j]);  // decoder gradient of this chunk's 32 samples
+        if (lane == 0) atomicAdd(&s_ddec[l * F + j], dd_lj);
+        gr[j] = gpre * s_dec[l * F + j] * lw;
+      }
+      float w8[8];
+      corner_weights(cell, w8);
+      // runs of adjacent samples that share a cell are summed before scattering (hash_bwd_plan.cuh)
+      float v[8][F];
+#pragma unroll
+      for (int k8 = 0; k8 < 8; ++k8)
+#pragma unroll
+        for (int j = 0; j < F; ++j) v[k8][j] = w8[k8] * gr[j];
+      merge_runs_and_scatter<F>(plan, l, g.log2_size, q.x, q.y, q.z, scal, cell, v, act_static, lane, dtable, spread);
     }
   }
   __syncthreads();
@@ -331,15 +350,24 @@ extern "C" int nrb_proposal_bwd(const nrb_rays_t* rays, const nrb_grid_t* grid, 
   const int64_t N = rays->num_rays;
   if (N == 0) return NRB_OK;
   const PropGrid g = make_prop_grid(grid, decoder_w, actor_grids, actor_samples, actor_dtables);
-  const unsigned blocks = blocks_for(N, kPropWarps);
+  // Rays per block: the scatter phase deals the block's rays * S samples to its warps as chunks of 32, so they are
+  // taken as the smallest of 4, 8 and 16 rays for which that is a multiple of 4 x 32 (whole chunks, the same number for
+  // every warp): 4 when S % 32 == 0, 8 when S % 16 == 0 (S = 48: 3 chunks per warp), 16 when S % 8 == 0.  Any other S
+  // keeps 4 rays and a partly filled last chunk.
+  int rays_per_block = kPropWarps;
+  while (rays_per_block < 4 * kPropWarps && (rays_per_block * iv->num_samples) % (kPropWarps * 32) != 0) rays_per_block *= 2;
+  if ((rays_per_block * iv->num_samples) % (kPropWarps * 32) != 0) rays_per_block = kPropWarps;
+  const unsigned blocks = blocks_for(N, rays_per_block);
+  const size_t smem = static_cast<size_t>(rays_per_block) * iv->num_samples * sizeof(float);  // at most 16 KB
   auto s = static_cast<cudaStream_t>(stream);
   BwdPlan plan;
   int64_t vertices = 0;
   if (int rc = prepare_bwd_plan(grid, N * iv->num_samples, workspace, workspace_bytes, s, &plan, &vertices)) return rc;
-#define NRB_LAUNCH_C(F, CH)                                                                                        \
-  proposal_bwd_kernel<F, CH><<<blocks, kPropWarps * 32, 0, s>>>(g, plan, rays->origins, rays->directions,          \
-                                                                rays->pixel_area, static_scale, *iv, N, saved_feats, \
-                                                                saved_pre, dweights, ddensity, dtable, ddecoder_w)
+#define NRB_LAUNCH_C(F, CH)                                                                                          \
+  proposal_bwd_kernel<F, CH><<<blocks, kPropWarps * 32, smem, s>>>(g, plan, rays->origins, rays->directions,         \
+                                                                   rays->pixel_area, static_scale, *iv, N,           \
+                                                                   rays_per_block, saved_feats, saved_pre, dweights, \
+                                                                   ddensity, dtable, ddecoder_w)
 #define NRB_LAUNCH(F)                                   \
   if (iv->num_samples <= 64) {                          \
     NRB_LAUNCH_C(F, 2);                                 \
