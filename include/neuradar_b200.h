@@ -223,6 +223,16 @@ int nrb_actor_assign(const nrb_rays_t* rays, const nrb_intervals_t* iv, const fl
  * [M,3] (optional) receives the gradient with respect to pos. */
 int nrb_actor_scatter(const nrb_actor_grids_t* grids, float* const* dtables, const nrb_actor_samples_t* samples,
                       const float* dyimg, float* dpos, int64_t M, nrb_stream_t stream);
+/* Gradient of the actor samples' features with respect to the world-to-box poses, for trained actor trajectories
+ * (NeuRADHashEncoding keeps grad mode for them, neurad_encoding.py:176-229; the box-frame point is
+ * transform_points_pairwise, cameras/lidars.py:507-519).  Inputs are those of the nrb_actor_assign call that produced
+ * `samples` - rays, iv, world2boxes [N,A,3,4], num_actors, flip [N] or NULL, actor_scale - plus its actor_index [M]
+ * output (M = N * iv->num_samples), the actor grids and dyimg, the tile image of d loss / d feature that
+ * nrb_actor_scatter reads.  dworld2boxes [N,A,3,4] += d loss / d world2boxes through the box-frame position, the flip,
+ * the contraction (mean and, outside its linear region, std) and the level weights.  No allocation, no synchronisation. */
+int nrb_actor_pose_grad(const nrb_rays_t* rays, const nrb_intervals_t* iv, const float* world2boxes, int32_t num_actors,
+                        const int32_t* actor_index, const float* flip, float actor_scale, const nrb_actor_grids_t* grids,
+                        const nrb_actor_samples_t* samples, const float* dyimg, float* dworld2boxes, nrb_stream_t stream);
 
 /* One linear layer y = x W^T + b (optional ReLU) through the same tcgen05 building blocks (K = 32 or 48,
  * n_out <= 48): the unit test of the descriptor / layout conventions. */

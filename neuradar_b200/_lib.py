@@ -145,6 +145,8 @@ SIGNATURES = {
     "nrb_hash_bwd_image": [C.POINTER(Grid), _P, _P, _P, _P, _P, _I64, _P, _I64, _P],
     "nrb_actor_assign": [C.POINTER(Rays), C.POINTER(Intervals), _P, _P, _P, _P, _I32, _P, _F, _P, _P, _P, _P, _P, _P],
     "nrb_actor_scatter": [C.POINTER(ActorGrids), C.POINTER(C.c_void_p), C.POINTER(ActorSamples), _P, _P, _I64, _P],
+    "nrb_actor_pose_grad": [C.POINTER(Rays), C.POINTER(Intervals), _P, _I32, _P, _P, _F, C.POINTER(ActorGrids),
+                            C.POINTER(ActorSamples), _P, _P, _P],
     "nrb_spaced_bins": [C.POINTER(Rays), Spacing, _P, _P, _I32, _I32, _P, _P, _P],
     "nrb_pdf_sample": [C.POINTER(Rays), Spacing, _P, _P, _I32, _P, _P, _I32, _F, _F, _P, _P, _P, _P, _P],
     "nrb_density_weights_fwd": [_P, C.POINTER(Intervals), _I64, _P, _P],

@@ -46,6 +46,16 @@ inline int check_actor_grids(const char* who, const nrb_actor_grids_t* g) {
   return NRB_OK;
 }
 
+// A world-space point in the frame of one actor box, m = world2boxes[n,a] [3,4] row-major: the rotation as a dot product,
+// then the translation (transform_points_pairwise, cameras/lidars.py:507-519).  Shared by the assignment and its
+// derivative, so that the pose gradient is taken at exactly the point the forward classified and contracted.
+__device__ __forceinline__ float3 to_box_frame(const float* m, const Gaussian& w) {
+  const float x = add(fmaf(m[2], w.z, fmaf(m[1], w.y, mul(m[0], w.x))), m[3]);
+  const float y = add(fmaf(m[6], w.z, fmaf(m[5], w.y, mul(m[4], w.x))), m[7]);
+  const float z = add(fmaf(m[10], w.z, fmaf(m[9], w.y, mul(m[8], w.x))), m[11]);
+  return make_float3(x, y, z);
+}
+
 // The 16 features of one actor sample (4 levels x 4 features, anti-alias weighted); the caller zero-pads to 32.
 __device__ __forceinline__ void actor_gather16(const ActorGridsDev& ag, int gid, float px, float py, float pz, float sd,
                                                float (&out)[16]) {

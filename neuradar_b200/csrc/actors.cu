@@ -77,11 +77,8 @@ __global__ void __launch_bounds__(256) actor_assign_kernel(const float* __restri
       bits &= bits - 1u;
       if (a >= A) break;
       if (!valid[n * A + a]) continue;
-      const float* m = world2boxes + (n * A + a) * 12;
-      // rotation as a dot product, then the translation (transform_points_pairwise, cameras/lidars.py:507-519)
-      const float x = add(fmaf(m[2], w.z, fmaf(m[1], w.y, mul(m[0], w.x))), m[3]);
-      const float y = add(fmaf(m[6], w.z, fmaf(m[5], w.y, mul(m[4], w.x))), m[7]);
-      const float z = add(fmaf(m[10], w.z, fmaf(m[9], w.y, mul(m[8], w.x))), m[11]);
+      const float3 b = to_box_frame(world2boxes + (n * A + a) * 12, w);
+      const float x = b.x, y = b.y, z = b.z;
       if (fabsf(x) < bounds[3 * a] && fabsf(y) < bounds[3 * a + 1] && fabsf(z) < bounds[3 * a + 2]) {
         hit = a;
         bx = x, by = y, bz = z;
@@ -151,6 +148,114 @@ __global__ void __launch_bounds__(256) actor_scatter_kernel(const __grid_constan
   }
 }
 
+// Gradient with respect to world2boxes [N,A,3,4] of the actor samples' features, for trained actor trajectories
+// (NeuRADHashEncoding keeps grad mode for the poses, neurad_encoding.py:176-229).  One thread per sample.  The sample's
+// box-frame point p = R x + t is recomputed with actor_assign_kernel's helper; its grid position and std are the
+// forward's own (`as`), so cells and level weights are the ones the forward used.  With g = d loss / d feat[0..15] (tile
+// image, as actor_scatter_kernel reads it):
+//   d pos = sum_l lw_l scal_l grad_o interp_l . g_l,   d std = sum_l lw_l'(std) interp_l . g_l,
+// lw_l' = -2 scal_l / (2 scal_l std)^2 where 2 scal_l std >= 1 (torch's clamp_min passes the gradient at equality), else
+// 0; then back through pos = (c + 2) / 4, std = sc / 4, the L-inf contraction of u = q / actor_scale (its full Jacobian
+// for the mean, and the sc(max|u|) path outside the linear region), the flip q = (f p_x, p_y, p_z) and p = R x + t:
+// dR += dp x^T, dt += dp.  The view direction takes no gradient (the SH encoding is no-grad).  The samples of one
+// (ray, actor) are consecutive, so a warp adds its lanes per key n * A + a (segmented scan) before the 12 atomics.
+__global__ void __launch_bounds__(256) actor_pose_grad_kernel(const float* __restrict__ origins,
+                                                              const float* __restrict__ directions,
+                                                              const float* __restrict__ pixel_area, nrb_intervals_t iv,
+                                                              const float* __restrict__ world2boxes, int A,
+                                                              const int32_t* __restrict__ actor_index,
+                                                              const float* __restrict__ flip, float actor_scale,
+                                                              const __grid_constant__ ActorGridsDev ag,
+                                                              const __grid_constant__ ActorSamplesDev as,
+                                                              const float* __restrict__ dyimg, float* __restrict__ dw2b,
+                                                              int64_t total) {
+  const int64_t gid = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const int lane = static_cast<int>(threadIdx.x) & (kWarp - 1);
+  const int hit = gid < total ? actor_index[gid] : -1;
+  if (__ballot_sync(kFull, hit >= 0) == 0u) return;  // (whole warps: the block size is a multiple of 32)
+  const int S = iv.num_samples;
+  const int64_t n = gid / S;
+  float g[12];
+#pragma unroll
+  for (int i = 0; i < 12; ++i) g[i] = 0.f;
+  if (hit >= 0) {
+    const int s = static_cast<int>(gid - n * S);
+    const Gaussian w = world_gaussian(origins[3 * n], origins[3 * n + 1], origins[3 * n + 2], directions[3 * n],
+                                      directions[3 * n + 1], directions[3 * n + 2], pixel_area[n],
+                                      iv.starts[n * iv.row_stride + s], iv.ends[n * iv.row_stride + s]);
+    const float3 p = to_box_frame(world2boxes + (n * A + hit) * 12, w);
+    const float f = flip != nullptr ? flip[n] : 1.0f;
+    // d loss / d (pos, std) of the 4-level lookup
+    const int grid = as.grid_id[gid];
+    const float px = as.pos[3 * gid], py = as.pos[3 * gid + 1], pz = as.pos[3 * gid + 2], sd = as.std[gid];
+    const uint32_t mask = (1u << ag.log2_size) - 1u;
+    float dpx = 0.f, dpy = 0.f, dpz = 0.f, dsd = 0.f;
+#pragma unroll
+    for (int l = 0; l < kActorLevels; ++l) {
+      const float scal = ag.scalings[l];
+      const Cell c = locate_cell(px, py, pz, scal, mask);
+      const float* base = ag.tables[grid] + (static_cast<size_t>(l) << ag.log2_size) * 4;
+      float gr[4], v[4];
+      load_row<4>(tile_image_chunk(dyimg, gid, l), 0, gr);
+      interpolate<4>(base, c, v);
+      const float t = mul(mul(scal, 2.0f), sd);
+      if (t >= 1.0f) dsd -= (gr[0] * v[0] + gr[1] * v[1] + gr[2] * v[2] + gr[3] * v[3]) * (2.0f * scal) / (t * t);
+      const float lw = level_weight(scal, sd);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) gr[j] *= lw;
+      const float3 d = position_grad<4>(base, c, gr);
+      dpx += d.x * scal, dpy += d.y * scal, dpz += d.z * scal;
+    }
+    // ... through pos = (c + 2) / 4, std = sc / 4 and contract_gaussian (the branch is the forward's: same fp32 u)
+    float dcx = 0.25f * dpx, dcy = 0.25f * dpy, dcz = 0.25f * dpz;
+    const float dsc = 0.25f * dsd;
+    const float ux = div(p.x * f, actor_scale), uy = div(p.y, actor_scale), uz = div(p.z, actor_scale);
+    const float ax = fabsf(ux), ay = fabsf(uy), az = fabsf(uz);
+    const float mag = fmaxf(fmaxf(ax, ay), az);
+    if (!(mag < 1.0f)) {
+      // c = h(m) u with h = 2/m - 1/m^2; sc = (std / scale) (2m - 1)^(2/3) / m^2; m = max |u_i| (torch's amax shares
+      // the gradient among tied maxima)
+      const float im = 1.0f / mag, h = (2.0f - im) * im, dh = 2.0f * im * im * (im - 1.0f);
+      const float q = cbrtf(2.0f * mag - 1.0f);
+      const float dr2 = (4.0f / 3.0f) / q * im * im - 2.0f * q * q * im * im * im;
+      const float dm = dh * (dcx * ux + dcy * uy + dcz * uz) + dsc * (w.std / actor_scale) * dr2;
+      const float ties = static_cast<float>((ax == mag) + (ay == mag) + (az == mag));
+      const float dmt = dm / ties;
+      dcx = h * dcx + (ax == mag ? (ux < 0.f ? -dmt : dmt) : 0.f);
+      dcy = h * dcy + (ay == mag ? (uy < 0.f ? -dmt : dmt) : 0.f);
+      dcz = h * dcz + (az == mag ? (uz < 0.f ? -dmt : dmt) : 0.f);
+    }
+    // ... through u = q / scale and the flip: d p
+    const float is = 1.0f / actor_scale;
+    const float dp[3] = {dcx * is * f, dcy * is, dcz * is};
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+      g[4 * r + 0] = dp[r] * w.x;
+      g[4 * r + 1] = dp[r] * w.y;
+      g[4 * r + 2] = dp[r] * w.z;
+      g[4 * r + 3] = dp[r];
+    }
+  }
+  // segmented inclusive sum over the warp's runs of equal (ray, actor); the last lane of a run adds it
+  const int64_t key = hit >= 0 ? n * A + hit : -1;
+  const int64_t prev = __shfl_up_sync(kFull, key, 1);
+  const int64_t next = __shfl_down_sync(kFull, key, 1);
+  const uint32_t heads = __ballot_sync(kFull, lane == 0 || prev != key);
+  const int head = 31 - __clz(heads & (0xFFFFFFFFu >> (31 - lane)));
+#pragma unroll
+  for (int o = 1; o < kWarp; o <<= 1) {
+#pragma unroll
+    for (int i = 0; i < 12; ++i) {
+      const float v = __shfl_up_sync(kFull, g[i], o);
+      if (lane - o >= head) g[i] += v;
+    }
+  }
+  if (hit >= 0 && (lane == kWarp - 1 || next != key)) {
+#pragma unroll
+    for (int i = 0; i < 12; ++i) atomicAdd(dw2b + key * 12 + i, g[i]);
+  }
+}
+
 }  // namespace nrb
 
 using namespace nrb;
@@ -195,4 +300,25 @@ extern "C" int nrb_actor_scatter(const nrb_actor_grids_t* grids, float* const* d
     actor_scatter_kernel<false><<<blocks_for(total, 256), 256, 0, s>>>(to_dev(grids), gd, as, dyimg, dpos, total);
   }
   return finish_launch("nrb_actor_scatter");
+}
+
+extern "C" int nrb_actor_pose_grad(const nrb_rays_t* rays, const nrb_intervals_t* iv, const float* world2boxes,
+                                   int32_t num_actors, const int32_t* actor_index, const float* flip, float actor_scale,
+                                   const nrb_actor_grids_t* grids, const nrb_actor_samples_t* samples, const float* dyimg,
+                                   float* dworld2boxes, nrb_stream_t stream) {
+  if (int rc = check_rays(rays)) return rc;
+  if (int rc = check_intervals("nrb_actor_pose_grad", iv)) return rc;
+  if (int rc = check_actor_grids("nrb_actor_pose_grad", grids)) return rc;
+  NRB_REQUIRE(world2boxes && actor_index && samples && samples->grid_id && samples->pos && samples->std && dyimg &&
+                  dworld2boxes,
+              NRB_ERR_BAD_ARG, "nrb_actor_pose_grad: null pointer");
+  NRB_REQUIRE(num_actors >= 1 && actor_scale > 0.f, NRB_ERR_BAD_ARG, "nrb_actor_pose_grad: bad num_actors / actor_scale");
+  NRB_REQUIRE(aligned16(dyimg), NRB_ERR_ALIGNMENT, "nrb_actor_pose_grad: dyimg must be 16-byte aligned");
+  if (rays->num_rays == 0) return NRB_OK;
+  const int64_t total = rays->num_rays * iv->num_samples;
+  const ActorSamplesDev as{samples->grid_id, samples->pos, samples->std, samples->dirs};
+  actor_pose_grad_kernel<<<blocks_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      rays->origins, rays->directions, rays->pixel_area, *iv, world2boxes, num_actors, actor_index, flip, actor_scale,
+      to_dev(grids), as, dyimg, dworld2boxes, total);
+  return finish_launch("nrb_actor_pose_grad");
 }

@@ -363,37 +363,51 @@ class NeuRADHashEncoding(nn.Module):
             return self.ray_flip_override
         return torch.bernoulli(torch.full((n,), self.config.actor.flip_prob, device=device)) * -2 + 1
 
+    def _poses_trainable(self) -> bool:
+        return any(p.requires_grad for p in getattr(self.actors, "parameters", lambda: [])())
+
     def can_assign_in_kernel(self, proposal: bool = False) -> bool:
         """The actor kernels cover the reference's default actor grids (4 levels, one table shape; 4 features in the field,
-        the static grid's feature count in a proposal network) for up to 32 actors, without gradients to the actor poses
-        (those take the torch bookkeeping below)."""
+        the static grid's feature count in a proposal network) for up to 32 actors.  Trained actor poses stay on them: the
+        field takes their gradient in CUDA (nrb_actor_pose_grad), and an encoding with require_actor_grad=False (the
+        proposal networks' default) treats them as constants, as the reference does.  A proposal network configured with
+        require_actor_grad=True and trained poses takes the torch bookkeeping below."""
         if not self.has_actors or len(self.actor_grids) == 0 or len(self.actor_grids) > 32:
             return False
         a = self.config.actor
         dim = self.config.static.hashgrid_dim if proposal else 4
         if proposal and self.config.static.num_levels < a.num_levels:
             return False
-        return a.num_levels == 4 and a.hashgrid_dim == dim and not any(
-            p.requires_grad for p in getattr(self.actors, "parameters", lambda: [])())
+        return a.num_levels == 4 and a.hashgrid_dim == dim and not (
+            proposal and self.config.require_actor_grad and self._poses_trainable())
 
-    @torch.no_grad()
     def assign_actors(self, rays: F.RayData, iv: F.SampleIntervals, times: Tensor) -> "F.ActorBatch":
-        """Which samples fall into which actor box, in one kernel (csrc/actors.cu): no nonzero(), no host synchronisation."""
+        """Which samples fall into which actor box, in one kernel (csrc/actors.cu): no nonzero(), no host synchronisation.
+        With trained poses, grad mode and require_actor_grad the batch carries the pose context (F.ActorPose), through
+        which the field differentiates with respect to the actor trajectories."""
+        track = torch.is_grad_enabled() and self._poses_trainable()
         key = (times.data_ptr(), times._version, tuple(times.shape))
         cached = None if self.pose_cache is None else self.pose_cache.get(key)
-        if cached is None:
-            boxes2world, valid = self.actors.get_boxes2world(times.reshape(-1), flatten=False)
-            # (R^T | -R^T t) element-wise: a matmul over [N, A] 3x3 blocks becomes A batched cuBLAS gemv launches
-            Ri = boxes2world[..., :3, :3].transpose(-2, -1)
-            world2boxes = torch.cat([Ri, -(Ri * boxes2world[..., None, :3, 3]).sum(-1, keepdim=True)], dim=-1).contiguous()
-            cached = (world2boxes, valid, times)  # (times is held so that its address cannot be recycled under the key)
+        # The encodings of one step share the cache and the proposal rounds fill it first: an entry always carries the
+        # graph when poses are trained, and an encoding that does not differentiate by them only reads it detached.
+        if cached is None or (track and not cached[0].requires_grad):
+            with torch.set_grad_enabled(track):
+                boxes2world, valid = self.actors.get_boxes2world(times.reshape(-1), flatten=False)
+                # (R^T | -R^T t) element-wise: a matmul over [N, A] 3x3 blocks becomes A batched cuBLAS gemv launches
+                Ri = boxes2world[..., :3, :3].transpose(-2, -1)
+                world2boxes = torch.cat([Ri, -(Ri * boxes2world[..., None, :3, 3]).sum(-1, keepdim=True)], dim=-1).contiguous()
+            cached = (world2boxes, valid.detach(), times)  # (times is held so that its address cannot be recycled under the key)
             if self.pose_cache is not None:
                 self.pose_cache[key] = cached
         world2boxes, valid = cached[0], cached[1]
+        pose_grad = track and self.config.require_actor_grad
         flip = self._draw_flip(rays.num_rays, rays.origins.device)
-        grid_id, pos, std, dirs = F.actor_assign(rays, iv, world2boxes, valid, self.actors.actor_bounds(), self.actors.actor_to_id,
-                                                 flip, self.actor_scale)
-        return F.ActorBatch(grid_id, pos, std, dirs, [g.hash_table for g in self.actor_grids], self.actor_grids[0].spec)
+        index = torch.empty((rays.num_rays * iv.num_samples,), device=rays.origins.device, dtype=torch.int32) if pose_grad else None
+        with torch.no_grad():
+            grid_id, pos, std, dirs = F.actor_assign(rays, iv, world2boxes, valid, self.actors.actor_bounds(),
+                                                     self.actors.actor_to_id, flip, self.actor_scale, index)
+        pose = F.ActorPose(world2boxes, index, flip, self.actor_scale, rays, iv) if pose_grad else None
+        return F.ActorBatch(grid_id, pos, std, dirs, [g.hash_table for g in self.actor_grids], self.actor_grids[0].spec, pose)
 
     @torch.no_grad()
     def _actor_indices(self, mean: Tensor, boxes2world: Tensor, valid: Tensor, world2boxes: Tensor, bounds: Tensor):

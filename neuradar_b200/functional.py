@@ -416,9 +416,24 @@ def _field_struct(weights: Sequence[Tensor], biases: Sequence[Optional[Tensor]],
 # dynamic actors: per-sample assignment (no compaction, no host synchronisation)
 # ------------------------------------------------------------------------------------------------
 @dataclass
+class ActorPose:
+    """What the pose gradient of an ActorBatch needs (nrb_actor_pose_grad): the inputs of the `actor_assign` call that
+    made the batch and its actor_index [M] int32 output.  `world2boxes` [N,A,3,4] carries the autograd graph back to the
+    actor trajectories; the field functions take it as an input and return its gradient."""
+
+    world2boxes: Tensor
+    actor_index: Tensor
+    flip: Optional[Tensor]
+    actor_scale: float
+    rays: RayData
+    iv: SampleIntervals
+
+
+@dataclass
 class ActorBatch:
     """Which samples of a [N,S] batch fall into which actor box (csrc/actors.cu): grid_id [M] int32 (-1 = static world),
-    pos [M,3] in the actor grid's unit cube, std [M], dirs [M,3] in the actor frame; plus the per-actor tables."""
+    pos [M,3] in the actor grid's unit cube, std [M], dirs [M,3] in the actor frame; plus the per-actor tables.  With a
+    `pose` the field functions also differentiate with respect to the actor poses."""
 
     grid_id: Tensor
     pos: Tensor
@@ -426,6 +441,7 @@ class ActorBatch:
     dirs: Tensor
     tables: List[Tensor]
     spec: GridSpec  # of ONE actor grid
+    pose: Optional[ActorPose] = None
 
     def grids_struct(self) -> "_lib.ActorGrids":
         g = _lib.ActorGrids()
@@ -454,9 +470,11 @@ class ActorBatch:
 
 
 def actor_assign(rays: RayData, iv: SampleIntervals, world2boxes: Tensor, valid: Tensor, bounds: Tensor, actor_to_id: Tensor,
-                 flip: Optional[Tensor], actor_scale: float) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                 flip: Optional[Tensor], actor_scale: float,
+                 actor_index: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """NeuRADHashEncoding._split_static_vs_actors as one kernel: (grid_id [M] int32, pos [M,3], std [M], dirs [M,3]) of the
-    M = N*S samples; world2boxes [N,A,3,4], valid [N,A], bounds [A,3], actor_to_id [A], flip [N] (+1 / -1) or None."""
+    M = N*S samples; world2boxes [N,A,3,4], valid [N,A], bounds [A,3], actor_to_id [A], flip [N] (+1 / -1) or None.
+    `actor_index` ([M] int32, optional) receives the index of each sample's actor in the ray's list (-1: none)."""
     N, S = rays.num_rays, iv.num_samples
     dev = rays.origins.device
     w2b = f32c(world2boxes.detach()[..., :3, :4])
@@ -470,7 +488,7 @@ def actor_assign(rays: RayData, iv: SampleIntervals, world2boxes: Tensor, valid:
     dirs = torch.zeros((N * S, 3), device=dev, dtype=torch.float32)
     r, i = rays.struct(), iv.struct()
     _lib.call("nrb_actor_assign", C.byref(r), C.byref(i), ptr(w2b), ptr(val), ptr(bnd), ptr(a2i), A, ptr(flp), float(actor_scale),
-              ptr(grid_id), ptr(pos), ptr(std), ptr(dirs), None, stream_ptr())
+              ptr(grid_id), ptr(pos), ptr(std), ptr(dirs), ptr(actor_index), stream_ptr())
     return grid_id, pos, std, dirs
 
 
@@ -479,8 +497,8 @@ def actor_assign(rays: RayData, iv: SampleIntervals, world2boxes: Tensor, valid:
 # ------------------------------------------------------------------------------------------------
 def _field_fused_backward(ctx, s: SimpleNamespace, dfeature, dfeat_ray, weights, dsdf, dalpha):
     """Shared by the two autograd Functions that end in the fused field kernel; `s` is `_saved(ctx)`.  Returns (dx or None,
-    the gradients of [table, beta, w0..w4, b0..b4, *actor tables] for autograd); in gather mode the hash-table gradient
-    is scattered here too."""
+    the gradients of [table, beta, w0..w4, b0..b4, *actor tables] for autograd, the gradient of the actor poses
+    world2boxes or None); in gather mode the hash-table gradient is scattered here too."""
     actors = None if ctx.actor_spec is None else ActorBatch.from_saved(s.actors, ctx.actor_spec)
     M, dev = s.sdf.shape[0], s.sdf.device
     need_dx = ctx.gather or ctx.needs_x_grad
@@ -519,13 +537,21 @@ def _field_fused_backward(ctx, s: SimpleNamespace, dfeature, dfeat_ray, weights,
         arr = (C.c_void_p * len(dactor))(*[ptr(t) for t in dactor])
         ag, asmp = actors.grids_struct(), actors.samples_struct()
         _lib.call("nrb_actor_scatter", C.byref(ag), arr, C.byref(asmp), ptr(dximg), None, M, stream_ptr())
-    return dx, sinks.written([dtable, *dmlp, *dactor])
+    dw2b = None
+    if ctx.pose is not None:  # trained actor poses: d loss / d world2boxes from the same feature gradient image
+        p = ctx.pose
+        dw2b = torch.zeros_like(p.world2boxes)
+        r, i = p.rays.struct(), p.iv.struct()
+        _lib.call("nrb_actor_pose_grad", C.byref(r), C.byref(i), ptr(p.world2boxes), p.world2boxes.shape[1],
+                  ptr(p.actor_index), ptr(p.flip), float(p.actor_scale), C.byref(ag), C.byref(asmp), ptr(dximg), ptr(dw2b),
+                  stream_ptr())
+    return dx, sinks.written([dtable, *dmlp, *dactor]), dw2b
 
 
 def _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, spec, beta, params, train,
-                         actors: Optional[ActorBatch] = None):
-    """Launch nrb_field_fused_fwd and set on ctx what the backward needs besides tensors.  Returns (feature, sdf, alpha,
-    the tensors to save by name or None when not training)."""
+                         actors: Optional[ActorBatch] = None, pose_grad: bool = False):
+    """Launch nrb_field_fused_fwd and set on ctx what the backward needs besides tensors (with `pose_grad`, the actor
+    batch's pose context).  Returns (feature, sdf, alpha, the tensors to save by name or None when not training)."""
     gather = table is not None
     ctx.sinks = _GradSinks([table, beta, *params])
     sh, beta = f32c(sh.detach()), f32c(beta)
@@ -558,6 +584,9 @@ def _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, 
               ptr(sdf), ptr(alpha), C.byref(sv), None if ag is None else C.byref(ag), None if asmp is None else C.byref(asmp),
               stream_ptr())
     ctx.actor_spec = None if actors is None else actors.spec
+    ctx.pose = None
+    if pose_grad:
+        ctx.pose = replace(actors.pose, world2boxes=f32c(actors.pose.world2boxes.detach()))
     ctx.samples_per_ray, ctx.beta_min, ctx.gather, ctx.spec = int(samples_per_ray), float(beta_min), gather, spec
     saved = None if not train else dict(
         table=table if gather else None, x3=x3 if gather else None, std=std if gather else None, ximg=ximg, masks=masks,
@@ -571,11 +600,11 @@ class _FieldFused(torch.autograd.Function):
 
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
-    def forward(ctx, table, x, x3, std, sh, samples_per_ray: int, beta_min: float, spec, actors, beta, *params):
+    def forward(ctx, table, x, x3, std, sh, samples_per_ray: int, beta_min: float, spec, actors, world2boxes, beta, *params):
         train = any(ctx.needs_input_grad)
         ctx.needs_x_grad = x is not None and ctx.needs_input_grad[1]
         feature, sdf, alpha, saved = _field_fused_forward(ctx, table, x, x3, std, sh, samples_per_ray, beta_min, spec, beta,
-                                                          params, train, actors)
+                                                          params, train, actors, ctx.needs_input_grad[9])
         if train:
             _save(ctx, **saved)
         return feature, sdf, alpha
@@ -587,8 +616,8 @@ class _FieldFused(torch.autograd.Function):
         dfeature = torch.zeros((s.sdf.shape[0], 32), device=s.sdf.device) if dfeature is None else f32c(dfeature)
         dsdf = None if dsdf is None else f32c(dsdf)
         dalpha = None if dalpha is None else f32c(dalpha)
-        dx, grads = _field_fused_backward(ctx, s, dfeature, None, None, dsdf, dalpha)
-        return (grads[0], dx, None, None, None, None, None, None, None, *grads[1:])
+        dx, grads, dw2b = _field_fused_backward(ctx, s, dfeature, None, None, dsdf, dalpha)
+        return (grads[0], dx, None, None, None, None, None, None, None, dw2b, *grads[1:])
 
 
 def field_fused(table: Optional[Tensor], x: Optional[Tensor], x3: Optional[Tensor], std: Optional[Tensor], sh: Tensor,
@@ -596,9 +625,16 @@ def field_fused(table: Optional[Tensor], x: Optional[Tensor], x3: Optional[Tenso
                 biases: Sequence[Optional[Tensor]], beta: Tensor, beta_min: float,
                 actors: Optional[ActorBatch] = None) -> Tuple[Tensor, Tensor, Tensor]:
     """Fused field.  Gather mode: `table` + sample means `x3` [M,3] + `std` [M] (+ `actors`: the samples inside actor boxes
-    read their actor's grid instead); otherwise hash features `x` [M,32]."""
+    read their actor's grid instead, and with `actors.pose` the actor poses get a gradient); otherwise hash features
+    `x` [M,32]."""
     extra = [] if actors is None else list(actors.tables)
-    return _FieldFused.apply(table, x, x3, std, sh, samples_per_ray, beta_min, spec, actors, beta, *weights, *biases, *extra)
+    return _FieldFused.apply(table, x, x3, std, sh, samples_per_ray, beta_min, spec, actors, _pose_input(actors), beta,
+                             *weights, *biases, *extra)
+
+
+def _pose_input(actors: Optional[ActorBatch]) -> Optional[Tensor]:
+    """The world2boxes input of the field Functions: present only with a pose context."""
+    return None if actors is None or actors.pose is None else actors.pose.world2boxes
 
 
 class _FieldRender(torch.autograd.Function):
@@ -609,12 +645,13 @@ class _FieldRender(torch.autograd.Function):
 
     @staticmethod
     @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
-    def forward(ctx, table, x3, std, sh, iv: "SampleIntervals", beta_min: float, spec, trans_eps: float, actors, beta, *params):
+    def forward(ctx, table, x3, std, sh, iv: "SampleIntervals", beta_min: float, spec, trans_eps: float, actors, world2boxes,
+                beta, *params):
         train = any(ctx.needs_input_grad)
         ctx.needs_x_grad = False
         S = iv.num_samples
         feature, sdf, alpha, saved = _field_fused_forward(ctx, table, None, x3, std, sh, S, beta_min, spec, beta, params, train,
-                                                          actors)
+                                                          actors, ctx.needs_input_grad[9])
         N, dev = alpha.shape[0] // S, alpha.device
         weights = torch.empty((N, S), device=dev, dtype=torch.float32)
         features = torch.empty((N, 32), device=dev, dtype=torch.float32)
@@ -642,8 +679,8 @@ class _FieldRender(torch.autograd.Function):
         i = ctx.iv.struct()
         _lib.call("nrb_alpha_composite_bwd", ptr(s.alpha), ptr(s.feature), C.byref(i), N, 32, ctx.trans_eps, 1, ptr(dweights),
                   ptr(dfeatures), ptr(ddepth), ptr(dacc), ptr(dalphas), None, stream_ptr())
-        _, grads = _field_fused_backward(ctx, s, None, dfeatures, s.render_weights.reshape(-1), None, dalphas)
-        return (grads[0], None, None, None, None, None, None, None, None, *grads[1:])
+        _, grads, dw2b = _field_fused_backward(ctx, s, None, dfeatures, s.render_weights.reshape(-1), None, dalphas)
+        return (grads[0], None, None, None, None, None, None, None, None, dw2b, *grads[1:])
 
 
 def field_render(table: Tensor, x3: Tensor, std: Optional[Tensor], sh: Tensor, iv: SampleIntervals, spec: GridSpec,
@@ -651,7 +688,8 @@ def field_render(table: Tensor, x3: Tensor, std: Optional[Tensor], sh: Tensor, i
                  trans_eps: float = 0.0, actors: Optional[ActorBatch] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """(weights [N,S], features [N,32], depth [N], accumulation [N]) of the rays whose samples are (x3, std, iv)."""
     extra = [] if actors is None else list(actors.tables)
-    return _FieldRender.apply(table, x3, std, sh, iv, beta_min, spec, trans_eps, actors, beta, *weights, *biases, *extra)
+    return _FieldRender.apply(table, x3, std, sh, iv, beta_min, spec, trans_eps, actors, _pose_input(actors), beta, *weights,
+                              *biases, *extra)
 
 
 def sh16(directions: Tensor, normalize_to_unit_cube: bool = False) -> Tensor:

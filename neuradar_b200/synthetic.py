@@ -120,9 +120,10 @@ class SyntheticActors(torch.nn.Module):
     NeuRADHashEncoding uses: `n_actors`, `get_boxes2world(times, flatten=False) -> ([N,A,4,4], valid [N,A])`,
     `actor_bounds() -> [A,3]`, `actor_to_id [A]`.  Actors are non-overlapping boxes on a grid around the origin that move on
     straight lines with a slow yaw (SURVEY.md 8d, config 4); poses are closed-form in time, as trajectory interpolation is
-    outside the hot path."""
+    outside the hot path.  With `trainable` the trajectory (`centres`, `velocity`, `yaw0`, `yaw_rate`) is made of
+    parameters under the same state-dict names, as the reference optimises its actor trajectories."""
 
-    def __init__(self, n_actors: int = 16, device: str = "cpu", seed: int = 5):
+    def __init__(self, n_actors: int = 16, device: str = "cpu", seed: int = 5, trainable: bool = False):
         super().__init__()
         g = torch.Generator().manual_seed(seed)
         self.n_actors = n_actors
@@ -131,10 +132,17 @@ class SyntheticActors(torch.nn.Module):
         # centres on a 12 m lattice inside the +-20 m area the synthetic rays start in; half extents of a car
         centres = torch.stack([(idx % side).float() * 12.0 - 6.0 * (side - 1), (idx // side).float() * 12.0 - 6.0 * (side - 1),
                                torch.full((n_actors,), 0.9)], -1)
-        self.register_buffer("centres", centres.to(device))
-        self.register_buffer("velocity", ((torch.rand((n_actors, 3), generator=g) - 0.5) * torch.tensor([0.2, 0.2, 0.0])).to(device))
-        self.register_buffer("yaw0", (torch.rand((n_actors,), generator=g) * 2 * math.pi).to(device))
-        self.register_buffer("yaw_rate", ((torch.rand((n_actors,), generator=g) - 0.5) * 0.02).to(device))
+        trajectory = dict(
+            centres=centres,
+            velocity=(torch.rand((n_actors, 3), generator=g) - 0.5) * torch.tensor([0.2, 0.2, 0.0]),
+            yaw0=torch.rand((n_actors,), generator=g) * 2 * math.pi,
+            yaw_rate=(torch.rand((n_actors,), generator=g) - 0.5) * 0.02,
+        )
+        for name, value in trajectory.items():
+            if trainable:
+                self.register_parameter(name, torch.nn.Parameter(value.to(device)))
+            else:
+                self.register_buffer(name, value.to(device))
         self.register_buffer("bounds", torch.tensor([1.0, 2.3, 0.85]).repeat(n_actors, 1).to(device))
         self.register_buffer("actor_to_id", torch.arange(n_actors).to(device))
         self.register_buffer("bottom_row", torch.tensor([0.0, 0.0, 0.0, 1.0]).to(device))
