@@ -33,7 +33,7 @@ extern "C" {
 #define NRB_MAX_MLP_LAYERS 4
 #define NRB_MAX_MLP_WIDTH 64
 #define NRB_MAX_SAMPLES 256 /* samples per ray handled by the warp-per-ray kernels */
-#define NRB_MAX_ACTORS 32   /* per-actor hash grids handled by the fused kernels */
+#define NRB_MAX_ACTORS 256  /* per-actor hash grids handled by the fused kernels */
 
 typedef void* nrb_stream_t; /* cudaStream_t */
 
@@ -91,6 +91,8 @@ typedef struct {
 } nrb_spacing_t;
 
 int nrb_version(void);
+/* NRB_MAX_ACTORS of this build: the length of nrb_actor_grids_t::tables, so that a binding can check its mirror. */
+int32_t nrb_max_actors(void);
 const char* nrb_last_error_string(void);
 /* Number of kernels this library has launched in the calling process (bench.py's gpu_launches). */
 int64_t nrb_launch_count(void);
@@ -156,7 +158,10 @@ typedef struct {
  * neurad_encoding.py:112-119,295-307).  tables[i] = actor_grids.i.hash_table [4 * 2^log2_hashmap_size, 4]; scalings = the
  * four level resolutions.  The per-sample assignment comes from nrb_actor_assign: grid_id [M] (-1 = static world), pos
  * [M,3] in the grid's unit cube, std [M], dirs [M,3] (view direction in the actor frame).  Samples with grid_id >= 0 take
- * their 16 features from that grid (zero-padded to 32, neurad_encoding.py:181-187) and the SH basis of dirs. */
+ * their 16 features from that grid (zero-padded to 32, neurad_encoding.py:181-187) and the SH basis of dirs.
+ * num_grids is 1..NRB_MAX_ACTORS (256); only tables[0 .. num_grids-1] are read.  Every entry point that takes actor grids
+ * returns NRB_ERR_UNSUPPORTED for more, before any launch.  The struct is passed to the kernels by value as part of their
+ * parameters (two such pointer arrays, 4 KB, in the proposal backward), which CUDA >= 12.1 allows on sm_100. */
 typedef struct {
   const float* tables[NRB_MAX_ACTORS];
   float scalings[NRB_MAX_LEVELS];

@@ -88,7 +88,7 @@ class FieldFusedBwdIn(C.Structure):
     ]
 
 
-MAX_ACTORS = 32
+MAX_ACTORS = 256  # NRB_MAX_ACTORS: the length of ActorGrids.tables, checked against the library in load()
 
 
 class ActorGrids(C.Structure):  # nrb_actor_grids_t
@@ -122,6 +122,7 @@ _F = C.c_float
 # name -> argtypes; every function returns int unless listed in _RESTYPES.  Mirrors include/neuradar_b200.h.
 SIGNATURES = {
     "nrb_version": [],
+    "nrb_max_actors": [],
     "nrb_last_error_string": [],
     "nrb_launch_count": [],
     "nrb_hash_fwd": [C.POINTER(Grid), _P, _P, _P, _I64, _P],
@@ -167,7 +168,7 @@ SIGNATURES = {
     "nrb_proposal_bwd": [C.POINTER(Rays), C.POINTER(Grid), _P, _F, C.POINTER(Intervals), _P, _P, _P, _P, _P, _P, _P, _I64,
                          C.POINTER(ActorGrids), C.POINTER(ActorSamples), C.POINTER(C.c_void_p), _P],
 }
-_RESTYPES = {"nrb_last_error_string": C.c_char_p, "nrb_launch_count": C.c_int64, "nrb_hash_bwd_workspace_bytes": C.c_int64, "nrb_field_saved_ld": C.c_int64,
+_RESTYPES = {"nrb_max_actors": C.c_int32, "nrb_last_error_string": C.c_char_p, "nrb_launch_count": C.c_int64, "nrb_hash_bwd_workspace_bytes": C.c_int64, "nrb_field_saved_ld": C.c_int64,
              "nrb_field_fused_image_bytes": C.c_int64}
 
 _lib: Optional[C.CDLL] = None
@@ -192,6 +193,9 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)  # AttributeError here means header and library disagree
         fn.argtypes = argtypes
         fn.restype = _RESTYPES.get(name, C.c_int)
+    if lib.nrb_max_actors() != MAX_ACTORS:  # every ActorGrids field after `tables` would be misplaced
+        raise NeuradarB200Error(f"{LIB_PATH} was built with NRB_MAX_ACTORS = {lib.nrb_max_actors()}, the binding expects "
+                                f"{MAX_ACTORS}; rebuild it with `python -m neuradar_b200.build`")
     _lib = lib
     return lib
 

@@ -28,19 +28,21 @@ __global__ void __launch_bounds__(256) actor_assign_kernel(const float* __restri
                                                            int64_t total) {
   // Per-ray pre-cull (the reference's own first filter, neurad_encoding.py:231-247): an actor can only claim samples of
   // a ray whose line passes its bounding sphere.  The block's 256 consecutive samples belong to a handful of rays; the
-  // first threads test every (ray, actor) pair once and leave a bit mask per ray, the per-sample loop below then runs
-  // the exact box test only for the flagged actors (typically none or one of 16).  The sphere contains the box, and the
-  // test is evaluated with a margin, so the result is the plain loop's.
-  constexpr int kCullRays = 8;
-  __shared__ uint32_t s_mask[kCullRays];
+  // block first tests every (ray, actor) pair once and leaves a bit set of ceil(A / 32) words per ray in shared memory
+  // (sized by the launch from S and A, actor_cull_bytes), and the per-sample loop below runs the exact box test only for
+  // the flagged actors (typically none or one).  The sphere contains the box, and the test is evaluated with a margin,
+  // so the result is the plain loop's.  Above NRB_MAX_ACTORS the launch passes no shared memory and every sample runs
+  // the plain loop.
+  extern __shared__ uint32_t s_mask[];  // [rays of the block][words]
   const int S = iv.num_samples;
   const int64_t first = static_cast<int64_t>(blockIdx.x) * blockDim.x;
   const int64_t last = min(first + blockDim.x, total) - 1;
   const int64_t n0 = first / S;
   const int nrays = static_cast<int>(last / S - n0) + 1;
-  const bool cull = nrays <= kCullRays && A <= 32;
+  const bool cull = A <= NRB_MAX_ACTORS;
+  const int words = (A + 31) / 32;
   if (cull) {
-    if (threadIdx.x < kCullRays) s_mask[threadIdx.x] = 0u;
+    for (int i = threadIdx.x; i < nrays * words; i += blockDim.x) s_mask[i] = 0u;
     __syncthreads();
     for (int p = threadIdx.x; p < nrays * A; p += blockDim.x) {
       const int64_t n = n0 + p / A;
@@ -56,7 +58,7 @@ __global__ void __launch_bounds__(256) actor_assign_kernel(const float* __restri
       const float cx = py * qz - pz * qy, cy = pz * qx - px * qz, cz = px * qy - py * qx;  // |p x q| = distance * |q|
       const float r2 = bounds[3 * a] * bounds[3 * a] + bounds[3 * a + 1] * bounds[3 * a + 1] + bounds[3 * a + 2] * bounds[3 * a + 2];
       if (cx * cx + cy * cy + cz * cz <= (r2 * 1.01f + 1.0e-6f) * (qx * qx + qy * qy + qz * qz))
-        atomicOr(&s_mask[p / A], 1u << a);
+        atomicOr(&s_mask[(p / A) * words + a / 32], 1u << (a % 32));
     }
     __syncthreads();
   }
@@ -69,21 +71,21 @@ __global__ void __launch_bounds__(256) actor_assign_kernel(const float* __restri
                                     iv.starts[n * iv.row_stride + s], iv.ends[n * iv.row_stride + s]);
   int hit = -1;
   float bx = 0.f, by = 0.f, bz = 0.f;
-  uint32_t todo = cull ? s_mask[n - n0] : (A >= 32 ? 0xFFFFFFFFu : (1u << A) - 1u);
-  for (int a0 = 0; a0 < A; a0 += 32) {  // (more than 32 actors: plain loop in chunks of 32)
-    uint32_t bits = a0 == 0 ? todo : 0xFFFFFFFFu;
-    while (bits != 0u) {
-      const int a = a0 + __ffs(bits) - 1;
-      bits &= bits - 1u;
-      if (a >= A) break;
-      if (!valid[n * A + a]) continue;
-      const float3 b = to_box_frame(world2boxes + (n * A + a) * 12, w);
-      const float x = b.x, y = b.y, z = b.z;
-      if (fabsf(x) < bounds[3 * a] && fabsf(y) < bounds[3 * a + 1] && fabsf(z) < bounds[3 * a + 2]) {
-        hit = a;
-        bx = x, by = y, bz = z;
-      }
+  auto box_test = [&](int a) {  // ascending a: the highest actor index wins
+    if (!valid[n * A + a]) return;
+    const float3 b = to_box_frame(world2boxes + (n * A + a) * 12, w);
+    if (fabsf(b.x) < bounds[3 * a] && fabsf(b.y) < bounds[3 * a + 1] && fabsf(b.z) < bounds[3 * a + 2]) {
+      hit = a;
+      bx = b.x, by = b.y, bz = b.z;
     }
+  };
+  if (cull) {
+    const uint32_t* flagged = s_mask + (n - n0) * words;
+    for (int k = 0; k < words; ++k) {
+      for (uint32_t bits = flagged[k]; bits != 0u; bits &= bits - 1u) box_test(32 * k + __ffs(bits) - 1);
+    }
+  } else {
+    for (int a = 0; a < A; ++a) box_test(a);
   }
   grid_id[gid] = hit >= 0 ? actor_to_id[hit] : -1;
   if (actor_index != nullptr) actor_index[gid] = hit;
@@ -100,6 +102,13 @@ __global__ void __launch_bounds__(256) actor_assign_kernel(const float* __restri
   pos[3 * gid] = c.x, pos[3 * gid + 1] = c.y, pos[3 * gid + 2] = c.z;
   std[gid] = c.std;
   dirs[3 * gid] = rx, dirs[3 * gid + 1] = ry, dirs[3 * gid + 2] = rz;
+}
+
+// Shared memory of actor_assign_kernel's pre-cull: the rays a block of 256 consecutive samples can touch (at most
+// ceil(255 / S) + 1, 256 for S = 1) times ceil(A / 32) mask words; at most 8 KB.  None above NRB_MAX_ACTORS.
+static size_t actor_cull_bytes(int S, int A) {
+  if (A > NRB_MAX_ACTORS) return 0;
+  return sizeof(uint32_t) * static_cast<size_t>((255 + S - 1) / S + 1) * ((A + 31) / 32);
 }
 
 struct ActorGradDev {
@@ -271,7 +280,8 @@ extern "C" int nrb_actor_assign(const nrb_rays_t* rays, const nrb_intervals_t* i
   NRB_REQUIRE(num_actors >= 1 && actor_scale > 0.f, NRB_ERR_BAD_ARG, "nrb_actor_assign: bad num_actors / actor_scale");
   if (rays->num_rays == 0) return NRB_OK;
   const int64_t total = rays->num_rays * iv->num_samples;
-  actor_assign_kernel<<<blocks_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+  actor_assign_kernel<<<blocks_for(total, 256), 256, actor_cull_bytes(iv->num_samples, num_actors),
+                        static_cast<cudaStream_t>(stream)>>>(
       rays->origins, rays->directions, rays->pixel_area, *iv, world2boxes, valid, bounds, actor_to_id, num_actors, flip,
       actor_scale, grid_id, pos, std, dirs, actor_index, total);
   return finish_launch("nrb_actor_assign");

@@ -92,5 +92,7 @@ int sm_count() {
 }  // namespace nrb
 
 extern "C" int nrb_version(void) { return NRB_VERSION; }
+
+extern "C" int32_t nrb_max_actors(void) { return NRB_MAX_ACTORS; }
 extern "C" const char* nrb_last_error_string(void) { return nrb::g_error; }
 extern "C" int64_t nrb_launch_count(void) { return nrb::g_launches.load(std::memory_order_relaxed); }

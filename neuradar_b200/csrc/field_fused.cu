@@ -999,6 +999,9 @@ extern "C" int nrb_field_fused_fwd(const nrb_field_mlp_t* p, const nrb_grid_t* g
     NRB_REQUIRE(aligned16(x), NRB_ERR_ALIGNMENT, "nrb_field_fused_fwd: x must be 16-byte aligned");
   }
   NRB_REQUIRE(aligned16(sh) && aligned16(feature), NRB_ERR_ALIGNMENT, "nrb_field_fused_fwd: sh and feature must be 16-byte aligned");
+  if (actor_grids != nullptr) {
+    if (int rc = check_actor_grids("nrb_field_fused_fwd", actor_grids)) return rc;
+  }
   if (M == 0) return NRB_OK;
   FusedFwdArgs a{};
   a.xyz = xyz, a.std = std, a.x = x, a.sh = sh, a.samples_per_ray = samples_per_ray, a.M = M;
@@ -1010,7 +1013,6 @@ extern "C" int nrb_field_fused_fwd(const nrb_field_mlp_t* p, const nrb_grid_t* g
   }
   const bool actors = actor_grids != nullptr;
   if (actors) {
-    if (int rc = check_actor_grids("nrb_field_fused_fwd", actor_grids)) return rc;
     NRB_REQUIRE(grid != nullptr && actor_samples && actor_samples->grid_id && actor_samples->pos && actor_samples->std &&
                     actor_samples->dirs,
                 NRB_ERR_BAD_ARG, "nrb_field_fused_fwd: actors need the gather mode and all per-sample actor arrays");

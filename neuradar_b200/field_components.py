@@ -21,6 +21,7 @@ import numpy as np
 import torch
 from torch import Tensor, nn
 
+from . import _lib
 from . import functional as F
 from .rays import GaussiansStd
 
@@ -368,11 +369,11 @@ class NeuRADHashEncoding(nn.Module):
 
     def can_assign_in_kernel(self, proposal: bool = False) -> bool:
         """The actor kernels cover the reference's default actor grids (4 levels, one table shape; 4 features in the field,
-        the static grid's feature count in a proposal network) for up to 32 actors.  Trained actor poses stay on them: the
-        field takes their gradient in CUDA (nrb_actor_pose_grad), and an encoding with require_actor_grad=False (the
-        proposal networks' default) treats them as constants, as the reference does.  A proposal network configured with
-        require_actor_grad=True and trained poses takes the torch bookkeeping below."""
-        if not self.has_actors or len(self.actor_grids) == 0 or len(self.actor_grids) > 32:
+        the static grid's feature count in a proposal network) for up to _lib.MAX_ACTORS (256) actor grids.  Trained
+        actor poses stay on them: the field takes their gradient in CUDA (nrb_actor_pose_grad), and an encoding with
+        require_actor_grad=False (the proposal networks' default) treats them as constants, as the reference does.  A
+        proposal network configured with require_actor_grad=True and trained poses takes the torch bookkeeping below."""
+        if not self.has_actors or len(self.actor_grids) == 0 or len(self.actor_grids) > _lib.MAX_ACTORS:
             return False
         a = self.config.actor
         dim = self.config.static.hashgrid_dim if proposal else 4

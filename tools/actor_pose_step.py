@@ -1,13 +1,16 @@
-"""Step time of the config-4 workload (65 536 rays, 128 field samples, 2^22 main table, 16 dynamic actors) when the actor
-trajectories are trained, on three routes:
+"""Step time of the config-4 workload (65 536 rays, 128 field samples, 2^22 main table, --actors dynamic actors, 16 by
+default) when the actor trajectories are trained, on three routes:
   kernel  trained poses on the actor kernels (nrb_actor_assign, the fused kernels, nrb_actor_scatter, nrb_actor_pose_grad)
   torch   trained poses on the torch bookkeeping (`can_assign_in_kernel` forced False in all three encodings), which is
           where trained poses ran before the pose gradient kernel existed
   fixed   fixed poses on the actor kernels (what bench.py --config 4 measures)
 One step = forward + bench_loss + backward.  Eager for all three, and replayed as one CUDA graph for the two kernel
 routes (the torch route synchronises the host and cannot be captured).  CUDA events, `--warmup` steps per measurement,
-`--steps` timed steps, `--runs` runs with the routes alternating.  Writes `actor_pose_step.json` to --out.
-Usage: python tools/actor_pose_step.py --out /tmp/actor_pose"""
+`--steps` timed steps, `--runs` runs with the routes alternating.  Also recorded, because SyntheticActors spreads its boxes
+on a 12 m lattice and at large --actors most of them are far from the synthetic rays: the fraction of the field's samples
+inside a box, and the mean time of one nrb_actor_assign launch (torch.profiler, in a pass of its own after the timings).
+Writes `actor_pose_step.json` (`actor_pose_step_A<actors>.json` for other counts than 16) to --out.
+Usage: python tools/actor_pose_step.py --out /tmp/actor_pose [--actors 64]"""
 import argparse
 import json
 import os
@@ -26,6 +29,7 @@ ap.add_argument("--rays", type=int, default=0)
 ap.add_argument("--warmup", type=int, default=10)
 ap.add_argument("--steps", type=int, default=50)
 ap.add_argument("--runs", type=int, default=3)
+ap.add_argument("--actors", type=int, default=16, help="dynamic actors (one grid each)")
 args = ap.parse_args()
 assert torch.cuda.is_available(), "this measurement needs a CUDA device"
 w = WORKLOADS[4]
@@ -37,7 +41,7 @@ def build(trainable: bool, torch_route: bool):
     L, F, T, r0, r1 = w.main
     model = build_hot_path(log2_main=T, log2_prop=w.prop_log2, num_proposal_samples=w.proposal_samples,
                            num_nerf_samples=w.nerf_samples, main_levels=L, main_features=F, main_res=(r0, r1), seed=42,
-                           device=dev, actors=SyntheticActors(w.actors, device=dev, trainable=trainable))
+                           device=dev, actors=SyntheticActors(args.actors, device=dev, trainable=trainable))
     model.train()
     if torch_route:
         for h in [model.field.hashgrid] + [p.hashgrid for p in model.proposal_fields]:
@@ -111,16 +115,44 @@ for run in range(args.runs):
     order = cases if run % 2 == 0 else cases[::-1]
     for k, fn in order:
         result[k].append(round(timed(fn), 4))
+# samples of the field inside actor boxes: the field's own assignment of one kernel-route forward
+inside = {}
+field = routes["kernel"].field.hashgrid
+assign = field.assign_actors
+
+
+def counting_assign(rays, iv, times):
+    batch = assign(rays, iv, times)
+    inside["fraction"] = float((batch.grid_id >= 0).float().mean())
+    return batch
+
+
+field.assign_actors = counting_assign
+torch.manual_seed(1234)
+steps["kernel"]()
+field.assign_actors = assign
+# per-launch time of the assignment kernel (all three encodings' launches of a kernel-route step)
+with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+    for _ in range(5):
+        steps["kernel"]()
+    torch.cuda.synchronize()
+assign_us = [e for e in prof.key_averages() if "actor_assign_kernel" in e.key]
+assign_launch_us = round(assign_us[0].device_time_total / assign_us[0].count, 2) if assign_us else None
 q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                    capture_output=True, text=True).stdout.strip().splitlines()
 line = {
-    "workload": w.description + ", actor trajectories trained (SyntheticActors(trainable=True))",
+    "workload": (w.description.replace(f"{w.actors} dynamic actors", f"{args.actors} dynamic actors")
+                 + ", actor trajectories trained (SyntheticActors(trainable=True))"),
+    "actors": args.actors,
+    "field_samples_in_boxes": round(inside.get("fraction", float("nan")), 5),
+    "nrb_actor_assign_us_per_launch": assign_launch_us,
     "card": q[0] if q else torch.cuda.get_device_name(),
     "ms_per_step": {k: v for k, v in result.items()},
     "pose_grad_kernel_vs_torch_route_max_rel": pose_rel,
     "timing": f"CUDA events, {args.warmup} warm-up + {args.steps} timed steps per measurement, {args.runs} runs alternating",
 }
 os.makedirs(args.out, exist_ok=True)
-with open(os.path.join(args.out, "actor_pose_step.json"), "w") as fh:
+name = "actor_pose_step.json" if args.actors == 16 else f"actor_pose_step_A{args.actors}.json"
+with open(os.path.join(args.out, name), "w") as fh:
     json.dump(line, fh, indent=1)
 print(json.dumps(line))
